@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the masurvival step path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload 2v2|1v1_heal_only|ffa|ffa_lidar]
+                    [--workload 2v2|1v1_heal_only|ffa|ffa_lidar] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[2], the config the metric is quoted on:
 default 2v2 (A=4, teams, melee cd 40, B=4, H=4, shrinking safe zone), 16384
@@ -15,10 +15,20 @@ What is timed is the STATIONARY workload, whatever --steps/--warmup are: before
 the timed region every batch is pre-rolled `--preroll` (default 1500) untimed
 steps so that episode phases are de-synchronised (mean episode ~420 steps) and
 contacts, TOI events, melee hits, deaths, death-drops and in-kernel auto-resets
-all occur at their steady-state rates.  Then W warm-up steps, then R >= 5
-repeats of EXACTLY K steps, each repeat bracketed by barrier + synchronize and
-timed with CUDA events, MAX over ranks per repeat; `ms_per_step` is the MEDIAN
-repeat.  R is raised until the timed work exceeds 50 ms.
+all occur at their steady-state rates.  Then a fixed number of untimed steps
+that keep the device busy, W warm-up steps, and EXACTLY K timed steps: up to
+--repeats repeats of >= 20 steps, spread over 3 000 steps of the roll-out
+with untimed steps between them (the step time drifts over a few hundred
+steps), each bracketed by barrier + synchronize and timed with CUDA events,
+MAX over ranks per repeat; `ms_per_step` is the MEDIAN per-step time of the
+repeats.  Every step count depends on the arguments alone, so the same
+arguments give the same inputs on every run and every build.
+
+`--dump-outputs DIR` writes what the last timed step returned (observation
+tensors in the library's layout, rewards, dones, episode statistics) as
+DIR/<name>.npy in float32, for the environments listed in env_index.npy: all
+of them, or a fixed seeded sample that keeps the files under 64 MB.  Two
+builds run with the same arguments can be compared output for output.
 
 Prints ONE JSON line (rank 0).  `value` = agent-steps/s with actions already
 resident in HBM; `e2e` = the same through the host-buffer C-ABI call
@@ -44,18 +54,45 @@ METRIC = 'agent_steps_per_sec'
 UNIT = 'agent-steps/s'
 L2_BYTES = 126e6
 NB_CPU = 61   # pre-generated random action batches of the CPU arms (same cycling rule as the GPU arm)
+BUSY_STEPS = 2500      # untimed steps right before the timed repeats: >= 150 ms of work for every workload below on a B200
+SPAN_STEPS = 3000      # the timed repeats are spread over this many steps of the roll-out (see run_ours)
+MIN_REPEAT_STEPS = 20  # shorter repeats would time the barrier around them as much as the steps
+DUMP_BYTES = 64 << 20  # --dump-outputs: at most this many bytes of .npy files
 
-# BASELINE.json `configs` made concrete (SURVEY.md section 8d / BASELINE.md section 3)
+# BASELINE.json `configs` made concrete (SURVEY.md section 8d / BASELINE.md section 3).  `rotate`: independent
+# batches stepped round-robin so that their state + outputs exceed the 126 MB L2 (1.3x L2 over the library's
+# device bytes per batch); fixed here rather than derived from the build, so every build steps the same batches.
 WORKLOADS = {
-    '2v2': dict(variant='2v2', envs=16384, agents=4, kernel='k_step<4,4,4,4>',
+    '2v2': dict(variant='2v2', envs=16384, agents=4, rotate=3, kernel='k_step<4,4,4,4>',
                 label='configs[2]: default 2v2 (A=4 teams, melee cd40, B=4, H=4, safe zone), random actions, auto-reset'),
-    '1v1_heal_only': dict(variant='1v1_heal_only', envs=4096, agents=2, kernel='k_step<2,4,4,2>',
+    '1v1_heal_only': dict(variant='1v1_heal_only', envs=4096, agents=2, rotate=23, kernel='k_step<2,4,4,2>',
                           label='configs[1]: 1v1 heal-only (A=2, B=0, H=4, melee damage 0), random actions, auto-reset'),
-    'ffa': dict(variant='ffa', envs=8192, agents=8, kernel='k_step<8,8,16,8>',
+    'ffa': dict(variant='ffa', envs=8192, agents=8, rotate=3, kernel='k_step<8,8,16,8>',
                 label='configs[3]: free-for-all max (A=8, B=8 randomized, H=16, grid 8), 65536 envs across 8 GPUs = 8192 per GPU, auto-reset'),
-    'ffa_lidar': dict(variant='ffa_lidar', envs=32768, agents=8, kernel='k_step<8,8,16,8>',
+    'ffa_lidar': dict(variant='ffa_lidar', envs=32768, agents=8, rotate=2, kernel='k_step<8,8,16,8>',
                       label='configs[4]: ffa max + 32-ray lidar block (doubled rays), 32768 envs per GPU, auto-reset'),
 }
+
+
+def repeat_sizes(k, r):
+    """K timed steps as at most r repeats of >= MIN_REPEAT_STEPS steps (one if K is smaller), lengths within one"""
+    r = max(1, min(r, k // MIN_REPEAT_STEPS))
+    return [k // r + (i < k % r) for i in range(r)]
+
+
+def dump_sample(n, bytes_per_env, n_files):
+    """environments written by --dump-outputs: all n, or a fixed seeded sample that keeps n_files .npy files
+    (128-byte headers) within DUMP_BYTES"""
+    cap = max(1, (DUMP_BYTES - 128 * n_files) // bytes_per_env)
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, size=cap, replace=False))
+
+
+def write_dump(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def workload_config(name, auto_reset=True):
@@ -172,7 +209,7 @@ def run_ours(args):
     # than L2") and no flush kernel perturbs the timed region.
     envs = [make_env(0)]
     batch_bytes = envs[0].device_bytes()
-    ROT = args.rotate or int(min(32, max(2, math.ceil(1.3 * L2_BYTES / batch_bytes))))
+    ROT = args.rotate or int(min(32, max(2, math.ceil(W['rotate'] * W['envs'] / N))))
     envs += [make_env(r) for r in range(1, ROT)]
     for e_ in envs:
         e_.reset()
@@ -249,26 +286,40 @@ def run_ours(args):
     clk = ClockSampler(local)
     if not os.environ.get('BENCH_NO_SMI'):
         clk.start()
-    est = timed(dev_step, max(args.warmup, 3)) / max(args.warmup, 3)     # the W warm-up steps double as the duration estimate
-    R = int(max(args.repeats, math.ceil(60.0 / max(est * args.steps, 1e-6))))
-    # The step time of this workload drifts by up to +-20 % over a few hundred steps (it follows the longest TOI chain /
-    # largest island among the batch, and wedged agents stay wedged for a while): identical from run to run -- the
-    # roll-out is deterministic -- but a median over a short window lands in a slow or a fast stretch.  Time >= 3 000 steps.
-    R = int(max(R, math.ceil(3000.0 / max(args.steps, 1))))
-    R = min(R, 2000)
     # The host-side pauses above (stats read-back, sampler start) let the GPU idle for a few ms, after which
     # the first ~40 ms of work run up to 35 % slower (measured: 20-step repeats of 4.0, 3.5, 3.4, 3.1, 2.9, 2.9 ...
-    # ms, identical from run to run): keep the device busy for 150 ms right before the timed repeats.
-    for _ in range(int(math.ceil(150.0 / max(est, 1e-6)))):
+    # ms, identical from run to run): keep the device busy for >= 150 ms, then the W warm-up steps, right before the
+    # timed repeats.  A count of steps, not a time, so that the timed steps compute the same thing on every run.
+    for _ in range(BUSY_STEPS + args.warmup):
         dev_step()
-    l0 = sum(e_.kernel_launches() for e_ in envs)
-    torch.cuda.profiler.start()        # `ncu --profile-from-start off` captures exactly the timed repeats (no effect otherwise)
-    reps = [timed(dev_step, args.steps) for _ in range(R)]
+    # The step time of this workload drifts by up to +-20 % over a few hundred steps (it follows the longest TOI chain /
+    # largest island among the batch, and wedged agents stay wedged for a while): identical from run to run -- the
+    # roll-out is deterministic -- but one short window lands in a slow or a fast stretch.  So the K timed steps are cut
+    # into repeats spread over SPAN_STEPS steps of the roll-out, with untimed steps between them.
+    sizes = repeat_sizes(args.steps, args.repeats)
+    gap = math.ceil(max(0, SPAN_STEPS - args.steps) / (len(sizes) - 1)) if len(sizes) > 1 else 0
+    reps, timed_launches = [], 0
+    torch.cuda.profiler.start()        # `ncu --profile-from-start off` captures the timed repeats and the steps between them
+    for i, n in enumerate(sizes):
+        for _ in range(gap if i else 0):
+            dev_step()
+        l0 = sum(e_.kernel_launches() for e_ in envs)
+        reps.append(timed(dev_step, n))
+        timed_launches += sum(e_.kernel_launches() for e_ in envs) - l0
     torch.cuda.profiler.stop()
-    launches_per_rep = (sum(e_.kernel_launches() for e_ in envs) - l0) // R
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # what the last timed step returned, copied on the device before the arms below step the batches again
+        last = envs[(tick[0] - 1) % ROT]._h
+        names = list(env.obs_shapes()) + ['rewards', 'dones', 'episode_return', 'episode_length']
+        outs = {k: last.tensor(k) for k in names + [k for k in ('immune', 'br_over', 'br_results') if last.has_tensor(k)]}
+        idx = dump_sample(N, 4 + sum(4 * t[0].numel() for t in outs.values()), 1 + len(outs))
+        sel = torch.as_tensor(idx, device=dev)
+        dumped = {'env_index': idx, **{k: t.index_select(0, sel).to(torch.float32) for k, t in outs.items()}}
     clocks = clk.stop()
-    ms_per_step = float(np.median(reps)) / args.steps
+    ms_per_step = float(np.median([ms / n for ms, n in zip(reps, sizes)]))
     value = n_gpus * N * A / (ms_per_step * 1e-3)
+    R = min(2000, max(args.repeats, math.ceil(SPAN_STEPS / args.steps)))    # repeats of K steps of the arms below
 
     # ---- the same loop with CUDA events around every kernel (roofline numerator) ---------------
     for e_ in envs:
@@ -398,9 +449,12 @@ def run_ours(args):
         'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
         'config': config_block(args.workload, n_gpus, N),
         'tile_plan': env._h.tile_plan(),
-        'l2': f'{ROT} batches of {N} envs stepped round-robin ({ROT} x {batch_bytes / 1e6:.0f} MB of state+outputs > 126 MB L2): inputs larger than L2, no flush',
-        'timing': {'method': 'median over repeats of K steps; each repeat: barrier+sync, CUDA events, max over ranks',
-                   'repeats': R, 'timed_ms_total': float(np.sum(reps)), 'rep_ms_min': float(np.min(reps)), 'rep_ms_max': float(np.max(reps)),
+        'l2': f'{ROT} batches of {N} envs stepped round-robin ({ROT} x {batch_bytes / 1e6:.0f} MB of state+outputs '
+              f'{">" if ROT * batch_bytes > L2_BYTES else "<="} 126 MB L2): inputs larger than L2, no flush',
+        'timing': {'method': 'K timed steps in repeats spread over the roll-out; each repeat: barrier+sync, CUDA events, max over '
+                             'ranks; median of the repeats\' ms per step',
+                   'repeats': len(sizes), 'repeat_steps': sizes, 'untimed_steps_between_repeats': gap, 'timed_ms_total': float(np.sum(reps)),
+                   'rep_ms_min': float(np.min(reps)), 'rep_ms_max': float(np.max(reps)),
                    'rep_ms': [round(float(x), 4) for x in reps[:64]],
                    'preroll_steps_per_batch': args.preroll, 'rotating_batches': ROT,
                    'mean_episode_steps_in_timed_region': (tot_steps / tot_eps) if tot_eps else None,
@@ -430,7 +484,7 @@ def run_ours(args):
                                      '(device-resident: msv_step; e2e: step_host_async/_wait with pinned host buffers, the last results '
                                      'awaited inside the timed region), so the groups\' steps overlap and one group\'s slowest blocks no '
                                      'longer idle the other SMs'},
-        'gpu_launches': int(launches_per_rep),
+        'gpu_launches': int(timed_launches),
         'clocks': clocks,
         'roofline': {'bound': 'hbm', 'achieved': achieved, 'peak': peak, 'unit': 'GB/s', 'frac': achieved / peak,
                      'traffic': ctr.get('dram_bytes_per_launch'), 'kernel': W['kernel'], 'kernel_ms': kavg_ms,
@@ -452,6 +506,8 @@ def run_ours(args):
             c1 = {k: ref_python_baseline(k) for k in ('1v1_default', '2v2')}     # BASELINE.json configs[0]: 1 env, 1000 steps, demo.py loop
             if all(c1.values()):
                 line['cpu_baseline_config1'] = c1
+        if dumped is not None:
+            write_dump(args.dump_outputs, {k: v if isinstance(v, np.ndarray) else v.cpu().numpy() for k, v in dumped.items()})
         print(json.dumps(line))
     for e_ in envs:
         e_.close()
@@ -506,17 +562,17 @@ def run_reference(args):
         b.step(acts[(t * 7) % NB_CPU])
     for t in range(args.warmup):
         b.step(acts[(t * 7) % NB_CPU])
-    reps = []
-    R = max(args.repeats, 5)
-    for _ in range(R):
+    reps, t = [], 0                               # seconds per step of each repeat of the K timed steps
+    for n in repeat_sizes(args.steps, max(args.repeats, 5)):
         t0 = time.perf_counter()
-        for t in range(args.steps):
-            b.step(acts[(t * 7) % NB_CPU])
-        reps.append(time.perf_counter() - t0)
-        if sum(reps) > 60.0 and len(reps) >= 5:
-            break
+        for _ in range(n):
+            rewards, dones = b.step(acts[(t * 7) % NB_CPU])
+            t += 1
+        reps.append((time.perf_counter() - t0) / n)
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, {'env_index': np.arange(sample), 'rewards': rewards, 'dones': dones})
     b.close()
-    dt = float(np.median(reps))
+    dt = float(np.median(reps)) * args.steps
     value = sample * args.steps * A / dt
     cb = {'value': value, 'unit': UNIT, 'cores': threads, 'kind': 'port',
           'sample': f'{sample} envs per step (bounded sample of the {N}-env workload), {preroll}-step pre-roll, median of {len(reps)} repeats, '
@@ -538,6 +594,7 @@ def run_reference(args):
 
 
 def main():
+    sys.dont_write_bytecode = True    # the benchmark may run from a read-only tree: it writes nothing there
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
     ap.add_argument('--steps', type=int, default=200)
@@ -547,11 +604,14 @@ def main():
     ap.add_argument('--envs', type=int, default=0, help='environments per GPU (default: the workload\'s BASELINE count)')
     ap.add_argument('--seed', type=int, default=0)
     ap.add_argument('--preroll', type=int, default=1500, help='untimed steps per batch before the timed region (stationary episode mix)')
-    ap.add_argument('--repeats', type=int, default=15, help='minimum number of timed repeats of K steps (median reported; the step time drifts by a few % over hundreds of steps as wedged agents come and go, so the median wants more than a handful)')
-    ap.add_argument('--rotate', type=int, default=0, help='independent env batches stepped round-robin (0: enough to exceed L2)')
+    ap.add_argument('--repeats', type=int, default=15, help='at most this many repeats of >= 20 of the K timed steps (median reported; the step time drifts by a few % over hundreds of steps as wedged agents come and go, so the median wants more than a handful)')
+    ap.add_argument('--rotate', type=int, default=0, help='independent env batches stepped round-robin (0: the workload\'s count, scaled to --envs; enough to exceed L2)')
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-phase', action='store_true', help='skip the per-episode-phase timing')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step returned to DIR/<name>.npy (float32)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:
