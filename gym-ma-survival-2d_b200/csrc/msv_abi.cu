@@ -64,6 +64,7 @@ struct msv_handle {
   int64_t launches;
   ObsTable obs;
   ObsTable obs_term;         // auto_reset == 2: same table, writing the "terminal_<key>" tensors
+  DevOut O_term;             // auto_reset == 2: O with the lidar pointers on the "terminal_lidar_*" tensors
   int64_t exported;          // live DLPack exports
   std::string err;
 };
@@ -541,6 +542,12 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
         h->obs_term.keys[k].base = buf;
       }
     }
+    h->O_term = O;
+    if (cfg->auto_reset == 2 && L > 0) {   // the finished episode's last scan, written by a second k_lidar
+      if (dalloc(h, &h->O_term.lidar_frac, N * A * L) || dalloc(h, &h->O_term.lidar_hit, N * A * L)) {
+        g_err = h->err; msv_destroy(h); return MSV_ERR_ALLOC;
+      }
+    }
   }
   const int64_t n = num_envs, a = A, b = B, hh = H, s = Sw, l = L;
   reg(h, "agent", O.agent, 0, {n, a, s});
@@ -572,6 +579,10 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
       if (it == h->tensors.end()) continue;
       TensorInfo t = it->second; t.ptr = h->obs_term.keys[k].base;
       extra[std::string("terminal_") + names[k]] = t;
+    }
+    if (L > 0) {
+      extra["terminal_lidar_frac"] = h->tensors["lidar_frac"]; extra["terminal_lidar_frac"].ptr = h->O_term.lidar_frac;
+      extra["terminal_lidar_hit"] = h->tensors["lidar_hit"]; extra["terminal_lidar_hit"].ptr = h->O_term.lidar_hit;
     }
     for (auto& kv : extra) h->tensors[kv.first] = kv.second;
   }
@@ -689,6 +700,7 @@ static int launch(msv_handle* h, int which, const uint8_t* actions, void* stream
     CK(msv_launch(h->cap, 0, C0, h->S, h->O, actions, st));
     { int rc = readback(h, st); if (rc) return rc; }
     CK(msv_launch_obs(h->C, h->S, h->obs_term, h->AC, h->O.dones, st));
+    if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O_term, h->BC, h->HC, st)); h->launches++; }
     CK(msv_launch(h->cap, 4, h->C, h->S, h->O, nullptr, st));
     h->launches += 3;
   } else {

@@ -483,13 +483,13 @@ k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, c
 // it first stages the environment's bodies (scan order: boxes, box items, heals, walls, agents) as a
 // table in shared memory; each warp then culls the table against its agent's fan -- one body per lane,
 // range and (for fans narrower than a half plane) the two edge half-planes, conservatively -- and the
-// surviving bodies, still in scan order, are ray-tested by every lane.  The minimum fraction wins, ties go
-// to the first body in scan order, exactly like the sequential scan of the reference's callback.
+// surviving bodies are ray-tested by every lane.  The minimum fraction wins; of equal fractions the body
+// created first (smallest body sequence number) wins, as in the oracle's scan of the world's body list.
 #define LID_MAXB 64            // >= MSV_MAX_BOXES * 2 + MSV_MAX_HEALS + 4 + MSV_MAX_AGENTS = 44
-#define LID_W 8
+#define LID_W 9
 __global__ void __launch_bounds__(256)
 k_lidar(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, const __grid_constant__ DevOut O, int EB, int BC, int HC) {
-  extern __shared__ float lid_sm[];                  // [EB][LID_MAXB][LID_W]: kind, x, y, then r | hx, hy, ax, ay, rot (agents: r, angle)
+  extern __shared__ float lid_sm[];                  // [EB][LID_MAXB][LID_W]: kind, x, y, then r | hx, hy, ax, ay, rot (agents: r, angle); [8] body seq
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // (the next step's k_step may be waiting to become resident)
   const int A = C.A, L = C.lidar_n, N = C.N;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -509,18 +509,23 @@ k_lidar(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, 
         const float4 b0 = S.box0[b * N + e]; const int reh = (S.box1[b * N + e].y >> 1) & 1;
         SBox bx; sb_set_shape(bx, b0.z, b0.w, reh);
         t[0] = __int_as_float(b < nb ? KIND_BOX : KIND_NONE); t[1] = b0.x; t[2] = b0.y; t[3] = bx.hx; t[4] = bx.hy; t[5] = bx.ax; t[6] = bx.ay; t[7] = __int_as_float(bx.rot);
+        t[8] = __int_as_float(S.boxseq[b * N + e]);
       } else if (b < oH) {
         const float4 it = S.item0[(b - oI) * N + e];
         t[0] = __int_as_float(b - oI < ni ? KIND_ITEM : KIND_NONE); t[1] = it.x; t[2] = it.y; t[3] = C.item_r;
+        t[8] = __int_as_float(S.item1[(b - oI) * N + e].y);
       } else if (b < oW) {
         const float2 hh = S.heal[(b - oH) * N + e];
         t[0] = __int_as_float(b - oH < nh ? KIND_HEAL : KIND_NONE); t[1] = hh.x; t[2] = hh.y; t[3] = C.heal_r;
+        t[8] = __int_as_float(S.healseq[(b - oH) * N + e]);
       } else if (b < oA) {
         t[0] = __int_as_float(KIND_WALL); t[1] = C.walls[b - oW].px; t[2] = C.walls[b - oW].py; t[3] = __int_as_float(b - oW);
+        t[8] = __int_as_float(C.B0 + C.H0 + (b - oW));     // the walls and agents keep the sequence numbers of the reset
       } else {
         const float4 o = S.akin0[(b - oA) * N + e];
         const bool al = (__float_as_int(S.akin1[(b - oA) * N + e].w) & 1) != 0;
         t[0] = __int_as_float(al ? KIND_AGENT : KIND_NONE); t[1] = o.x; t[2] = o.y; t[3] = C.agent_r; t[4] = o.z;
+        t[8] = __int_as_float(C.B0 + C.H0 + 4 + (b - oA));
       }
     }
   }
@@ -581,7 +586,7 @@ k_lidar(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, 
       const float perp = off.x * dy - off.y * dx, along = off.x * dx + off.y * dy;
       return fabsf(perp) > lim || along < -lim || along > dd * dd + lim;
     };
-    float best = 2.0f; int bestb = -1;
+    float best = 2.0f; int bestb = -1, bestseq = 0;
     unsigned long long m = cand;
     while (m) {
       const int b = __ffsll((long long)m) - 1; m &= m - 1;
@@ -603,7 +608,7 @@ k_lidar(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, 
       } else {                                         // item, heal or agent circle
         if (!far_from(t[1], t[2], t[3] + 0.01f)) hit = ray_circle(mk2(t[1], t[2]), t[3], me, p2, f);
       }
-      if (hit && f < best) { best = f; bestb = b; }    // scan order is ascending b: strict < keeps the first of equal fractions
+      if (hit && (f < best || (f == best && __float_as_int(t[8]) < bestseq))) { best = f; bestb = b; bestseq = __float_as_int(t[8]); }
     }
     float fr = 1.0f; int hitcode = 0;
     if (bestb >= 0) {

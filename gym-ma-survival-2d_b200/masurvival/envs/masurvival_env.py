@@ -32,7 +32,10 @@ class MaSurvivalVec:
                             observation is then the first one of the new
                             episode (rewards/dones still describe the old).
                             'terminal': same, and step()'s info dict carries
-                            info['terminal_observation'] (rows valid where done)
+                            info['terminal_observation'] (rows valid where done),
+                            lidar_frac / lidar_hit included when lidars are
+                            configured (one more lidar scan per step, in this
+                            mode only)
     """
 
     metadata = {'render_modes': [], 'render_fps': 30}
@@ -112,8 +115,6 @@ class MaSurvivalVec:
         h, A = self._h, self.n_agents
         x = {}
         for k in self.obs_shapes():
-            if prefix and k.startswith('lidar'):
-                continue
             t = h.tensor(prefix + k)
             if k in ('zone', 'heals', 'boxes', 'box_items'):
                 t = t.unsqueeze(1).expand(t.shape[0], A, *t.shape[1:])
