@@ -787,6 +787,30 @@ int msv_step(msv_handle* h, const uint8_t* actions_dev, void* stream) {
   return launch(h, 0, actions_dev, stream);
 }
 
+int msv_render(msv_handle* h, int32_t first, int32_t count, int32_t height, int32_t width, uint32_t flags,
+               uint8_t* out_dev, void* stream) {
+  if (!h || !out_dev) return MSV_ERR_INVALID;
+  if (first < 0 || count < 1 || (int64_t)first + count > h->C.n_real || height < 1 || height > 4096 || width < 1 ||
+      width > 4096 || (flags & ~MSV_RENDER_LIDAR) || ((flags & MSV_RENDER_LIDAR) && h->C.lidar_n == 0)) {
+    h->err = "msv_render: env range, image size (1..4096) or flags out of range";
+    return MSV_ERR_INVALID;
+  }
+  DevGuard g(h->device);
+  RenderArgs R = {};
+  R.first = first; R.count = count; R.H = height; R.W = width; R.BC = h->BC; R.HC = h->HC;
+  R.lidar = (flags & MSV_RENDER_LIDAR) ? 1 : 0; R.out = out_dev;
+  const cudaError_t e = msv_launch_render(h->C, h->S, h->O, R, (cudaStream_t)stream);
+  h->launches++;
+  h->last_was_step = false;    // the next k_step must not wait for an observation kernel that is not the last launch
+  CK(e);
+  return MSV_OK;
+}
+
+int msv_render_palette(uint8_t* out_rgb, int32_t capacity) {
+  if (capacity < 0 || (capacity > 0 && !out_rgb)) return MSV_ERR_INVALID;
+  return msv_palette(out_rgb, capacity);
+}
+
 int msv_step_host_async(msv_handle* h, const uint8_t* actions_host, float* rewards_host, uint8_t* dones_host, void* obs_host,
                         void* stream) {
   if (!h || !actions_host) return MSV_ERR_INVALID;

@@ -1,5 +1,5 @@
 // msv_launch.h -- host-side interface between the C ABI (msv_abi.cu) and the
-// kernel launchers (msv_kernels.cu).
+// kernel launchers (msv_kernels.cu, msv_render.cu).
 #pragma once
 #include "msv_types.cuh"
 #ifndef MSV_TPB
@@ -18,3 +18,13 @@ cudaError_t msv_read_check(unsigned long long out[2]);
 cudaError_t msv_launch_spare(const DevConst& C, const DevState& S, const uint8_t* dones, int only_done, cudaStream_t st);
 cudaError_t msv_launch_obs(const DevConst& C, const DevState& S, const ObsTable& T, int AC, const uint8_t* only_if, cudaStream_t st);
 cudaError_t msv_launch_lidar(const DevConst& C, const DevState& S, const DevOut& O, int BC, int HC, cudaStream_t st);
+// msv_render: picture of envs [first, first+count) into out (uint8[count][H][W][3]); BC, HC the list capacities,
+// lidar != 0 draws the rays.  The launcher fills in the tiling and the viewport (the fields after `lidar`).
+struct RenderArgs {
+  int first, count, H, W, BC, HC, lidar;
+  int TW, TR, tiles_x, tiles_per_img;   // tile width and rows, tiles per image row and per image
+  float s, half_floor;                  // pixel size, floor_size / 2
+  uint8_t* out;
+};
+cudaError_t msv_launch_render(const DevConst& C, const DevState& S, const DevOut& O, RenderArgs R, cudaStream_t st);
+int msv_palette(uint8_t* out_rgb, int capacity);   // copies min(capacity, n) colours, returns n

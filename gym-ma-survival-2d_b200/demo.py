@@ -2,17 +2,25 @@
 """Headless counterpart of the reference's demo.py (demo.py:76-158, 164-293)
 for the batched B200 environment: random-policy rollout, optional JSON config
 (`-c`, same nested keys as the reference; shapes are given as radii), episode
-statistics (`flush_stats`) and the `--benchmark` per-step timing line.
-Rendering / interactive play are outside the accelerated path (SURVEY.md §2).
+statistics (`flush_stats`), the `--benchmark` per-step timing line, and a
+headless frame dumper (`--dump-frames DIR`): after every `--frame-every`-th
+step, a grid of the first `--frame-envs` environments drawn on the GPU
+(MaSurvivalVec.render) is written as DIR/frame_<step>.png.  Frames are drawn
+outside the timed window.  The pygame window and interactive play of the
+reference are not reproduced.
 
     python gym-ma-survival-2d_b200/demo.py -n 4096 --max-steps 1000 --benchmark
+    python gym-ma-survival-2d_b200/demo.py -n 16 --max-steps 200 --dump-frames frames --frame-envs 4
 """
 import argparse
 import json
+import math
 import os
 import pprint
+import struct
 import sys
 import time
+import zlib
 
 import numpy as np
 
@@ -37,8 +45,49 @@ class RandomPolicy:
         return a
 
 
-def demo_env(env, max_steps=None, print_benchmark=False, seed=0):
-    """Runs until every env finished one episode (auto_reset off) or max_steps."""
+def write_png(path, rgb):
+    """uint8[H, W, 3] -> PNG (8-bit RGB, one zlib stream, filter type 0 on every row); standard library only."""
+    h, w, _ = rgb.shape
+    raw = b''.join(b'\x00' + rgb[y].tobytes() for y in range(h))
+
+    def chunk(tag, data):
+        return struct.pack('>I', len(data)) + tag + data + struct.pack('>I', zlib.crc32(tag + data) & 0xffffffff)
+    with open(path, 'wb') as f:
+        f.write(b'\x89PNG\r\n\x1a\n' + chunk(b'IHDR', struct.pack('>IIBBBBB', w, h, 8, 2, 0, 0, 0))
+                + chunk(b'IDAT', zlib.compress(raw, 6)) + chunk(b'IEND', b''))
+
+
+class FrameDumper:
+    """Grid of the first `k` environments, ceil(sqrt(k)) per row, `size` pixels each: drawn and assembled
+    on the device, copied to the host once per frame."""
+
+    def __init__(self, env, out_dir, k=1, size=256, every=1):
+        import torch
+        if not 1 <= k <= env.num_envs:
+            raise ValueError(f'--frame-envs must be in 1..{env.num_envs}')
+        if every < 1:
+            raise ValueError('--frame-every must be >= 1')
+        self.env, self.dir, self.k, self.size, self.every = env, out_dir, k, size, every
+        self.cols = math.ceil(math.sqrt(k))
+        self.rows = math.ceil(k / self.cols)
+        dev = f'cuda:{env.device}'
+        self.frames = torch.empty((k, size, size, 3), dtype=torch.uint8, device=dev)
+        self.grid = torch.zeros((self.rows * self.cols, size, size, 3), dtype=torch.uint8, device=dev)
+        os.makedirs(out_dir, exist_ok=True)
+
+    def __call__(self, t):
+        if t % self.every:
+            return
+        self.env.render(count=self.k, height=self.size, width=self.size, out=self.frames)
+        self.grid[:self.k] = self.frames
+        S = self.size
+        img = self.grid.view(self.rows, self.cols, S, S, 3).permute(0, 2, 1, 3, 4).reshape(self.rows * S, self.cols * S, 3)
+        write_png(os.path.join(self.dir, f'frame_{t:05d}.png'), img.cpu().numpy())
+
+
+def demo_env(env, max_steps=None, print_benchmark=False, seed=0, dumper=None):
+    """Runs until every env finished one episode (auto_reset off) or max_steps; `dumper(t)` is called
+    after step t (1, 2, ...), outside the timed window."""
     import torch
     policy = RandomPolicy(env, seed)
     times = []
@@ -53,6 +102,8 @@ def demo_env(env, max_steps=None, print_benchmark=False, seed=0):
         times.append(time.perf_counter() - t0)
         done_once |= done
         t += 1
+        if dumper is not None:
+            dumper(t)
         if max_steps is not None and t == max_steps:
             print(f'Maximum number of steps {t} reached, terminating episode.')
             break
@@ -75,13 +126,20 @@ def main():
     ap.add_argument('-b', '--benchmark', action='store_true', help='print mean/std of the per-step time (demo.py:274-279)')
     ap.add_argument('--seed', type=int, default=0)
     ap.add_argument('--device', type=int, default=0)
+    ap.add_argument('--dump-frames', metavar='DIR', help='write a PNG of the first --frame-envs environments after steps')
+    ap.add_argument('--frame-envs', type=int, default=1, metavar='K', help='environments per frame, ceil(sqrt(K)) per row')
+    ap.add_argument('--frame-size', type=int, default=256, metavar='S', help='pixels per environment (S x S)')
+    ap.add_argument('--frame-every', type=int, default=1, metavar='T', help='a frame after every T-th step')
     args = ap.parse_args()
     config = None
     if args.config is not None:
         with open(args.config) as f:
             config = json.load(f)
     env = MaSurvivalVec(config, num_envs=args.num_envs, device=args.device, seed=args.seed, auto_reset=args.max_steps is not None)
-    demo_env(env, args.max_steps, args.benchmark, args.seed)
+    dumper = None
+    if args.dump_frames is not None:
+        dumper = FrameDumper(env, args.dump_frames, args.frame_envs, args.frame_size, args.frame_every)
+    demo_env(env, args.max_steps, args.benchmark, args.seed, dumper)
 
 
 if __name__ == '__main__':

@@ -22,12 +22,27 @@ EXPORTS = [
     'msv_step_host', 'msv_step_host_obs', 'msv_step_host_async', 'msv_step_host_wait', 'msv_obs_host_bytes',
     'msv_obs_host_offset', 'msv_device_bytes', 'msv_tensor', 'msv_tensor_info', 'msv_get_state', 'msv_set_state',
     'msv_observe', 'msv_flush_stats', 'msv_bytes_per_env_step', 'msv_kernel_bytes_per_env', 'msv_obs_bytes_per_env', 'msv_kernel_launches', 'msv_tile_plan', 'msv_plan_tile',
-    'msv_last_error', 'msv_philox4x32',
+    'msv_last_error', 'msv_philox4x32', 'msv_render', 'msv_render_palette',
 ]
+
+MSV_RENDER_LIDAR = 1
+# the entries of msv_render_palette(), in the library's order (include/masurv.h)
+RENDER_COLOURS = ('background', 'floor', 'floor_outside_zone', 'zone_ring', 'next_zone_ring', 'wall', 'heal',
+                  'box_item', 'box') + tuple(f'agent{i}' for i in range(8)) + ('team0', 'team1', 'heading', 'lidar_ray')
 
 
 class MasurvError(RuntimeError):
     pass
+
+
+def render_palette():
+    """The colours msv_render draws with: uint8[n, 3], row k is RENDER_COLOURS[k] (no device needed)."""
+    L = load()
+    out = np.zeros((64, 3), dtype=np.uint8)
+    n = L.msv_render_palette(out.ctypes.data, out.shape[0])
+    if n < 0:
+        check(n)
+    return out[:n].copy()
 
 
 _lib = None
@@ -84,6 +99,8 @@ def load():
     L.msv_last_error.argtypes = [vp]
     L.msv_last_error.restype = ctypes.c_char_p
     L.msv_philox4x32.argtypes = [vp, vp, vp]
+    L.msv_render.argtypes = [vp, i32, i32, i32, i32, ctypes.c_uint32, vp, vp]
+    L.msv_render_palette.argtypes = [vp, i32]
     L.msv_debug_step_kernel.argtypes = [vp, vp, vp]
     L.msv_debug_obs_kernel.argtypes = [vp, vp]
     L.msv_debug_overflow.argtypes = [vp]
@@ -167,6 +184,11 @@ class Handle:
 
     def observe_only(self, stream=0):
         check(load().msv_debug_obs_kernel(self.h, stream), self.h)
+
+    def render(self, first, count, out, flags=0, stream=0):
+        """msv_render into `out`, a contiguous CUDA uint8 tensor [count, H, W, 3] (the caller checks it)."""
+        check(load().msv_render(self.h, int(first), int(count), int(out.shape[1]), int(out.shape[2]), int(flags),
+                                out.data_ptr(), stream), self.h)
 
     def step_host(self, actions, rewards, dones, stream=0):
         check(load().msv_step_host(self.h, actions, rewards, dones, stream), self.h)

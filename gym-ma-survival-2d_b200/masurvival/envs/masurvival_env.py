@@ -38,7 +38,7 @@ class MaSurvivalVec:
                             mode only)
     """
 
-    metadata = {'render_modes': [], 'render_fps': 30}
+    metadata = {'render_modes': ['rgb_array'], 'render_fps': 30}
 
     def __init__(self, config=None, num_envs=1, device=0, seed=0, env_offset=0, auto_reset=True):
         self.config, self._continuous_melee = merge_config(config)
@@ -290,8 +290,27 @@ class MaSurvivalVec:
     def device_bytes(self):
         return self._h.device_bytes()
 
-    def render(self, mode='human'):
-        raise NotImplementedError('rendering is outside the accelerated step path (SURVEY.md section 2)')
+    def render(self, mode='rgb_array', first=0, count=None, height=256, width=256, lidar=False, out=None):
+        """Top-down RGB pictures of environments [first, first+count) as drawn by the library's
+        render kernel from the device state: a CUDA uint8 tensor [count, height, width, 3] (row 0 at
+        the top, +y up), enqueued on the current torch stream after the last step.  Under auto_reset,
+        a finished environment shows the first state of its new episode.  `lidar=True` draws the rays
+        (lidars must be configured).  Pass `out` (same shape, contiguous, on this device) to reuse a
+        buffer.  Colours: masurvival._lib.render_palette(), named by _lib.RENDER_COLOURS."""
+        import torch
+        if mode != 'rgb_array':
+            raise NotImplementedError(f'render mode {mode!r}: only rgb_array is supported (there is no window)')
+        count = self.num_envs - first if count is None else count
+        if count < 1 or height < 1 or width < 1:
+            raise ValueError(f'render: count, height and width must be positive (got {count}, {height}, {width})')
+        shape = (int(count), int(height), int(width), 3)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.uint8, device=f'cuda:{self.device}')
+        elif not (isinstance(out, torch.Tensor) and out.is_cuda and out.device.index == self.device
+                  and out.dtype == torch.uint8 and tuple(out.shape) == shape and out.is_contiguous()):
+            raise ValueError(f'out must be a contiguous uint8 tensor of shape {shape} on cuda:{self.device}')
+        self._h.render(first, count, out, _lib.MSV_RENDER_LIDAR if lidar else 0, self._stream())
+        return out
 
     def close(self):
         self._h.close()
@@ -311,6 +330,10 @@ class MaSurvival(MaSurvivalVec):
     def reset(self, seed=None, return_info=False, options=None):
         obs = self._np_obs(super().reset())
         return (obs, {}) if return_info else obs
+
+    def render(self, mode='rgb_array', height=256, width=256, lidar=False):
+        """numpy uint8[height, width, 3] picture of the environment (gym's rgb_array convention)."""
+        return super().render(mode, 0, 1, height, width, lidar)[0].cpu().numpy()
 
     def step(self, actions):
         actions = tuple(a for a in actions)

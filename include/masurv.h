@@ -310,6 +310,22 @@ int msv_set_state(msv_handle* h, int32_t first, int32_t count,
  * (fetch_observations, env:510-657), e.g. after msv_set_state. */
 int msv_observe(msv_handle* h, void* cuda_stream);
 
+/* Top-down RGB picture of envs [first, first+count), out_dev: device pointer to
+ * uint8[count][height][width][3] (row 0 at the top, +y up; the viewport is the
+ * floor and its walls with a margin of a wall's width, centred on the origin).
+ * Stream-ordered after everything already enqueued on cuda_stream (e.g. the
+ * msv_step whose result it shows); reads the state, writes only out_dev.
+ * height and width are 1..4096; MSV_RENDER_LIDAR needs lidars in the config.
+ * Colours are the entries of msv_render_palette, in this order: background,
+ * floor, floor outside the safe zone, zone ring, next-zone ring, wall, heal,
+ * box item, box, agent 0 .. agent 7, team 0, team 1, heading tick, lidar ray. */
+#define MSV_RENDER_LIDAR 1u   /* draw the lidar rays (only with lidars configured) */
+int msv_render(msv_handle* h, int32_t first, int32_t count, int32_t height, int32_t width,
+               uint32_t flags, uint8_t* out_dev, void* cuda_stream);
+/* Copies min(capacity, n) colours (3 bytes each) to out_rgb and returns n, the
+ * number of colours; out_rgb may be NULL when capacity is 0.  Needs no device. */
+int msv_render_palette(uint8_t* out_rgb, int32_t capacity);
+
 /* flush_stats (env:471-480) summed over all envs; zeroes the accumulators.
  * Synchronises the device first (work queued on any stream is complete). */
 int msv_flush_stats(msv_handle* h, msv_stats* out);
