@@ -65,6 +65,8 @@ struct msv_handle {
   ObsTable obs;
   ObsTable obs_term;         // auto_reset == 2: same table, writing the "terminal_<key>" tensors
   DevOut O_term;             // auto_reset == 2: O with the lidar pointers on the "terminal_lidar_*" tensors
+  uint8_t* truncated = nullptr;   // max_episode_steps > 0: the "truncated" tensor [N]
+  uint8_t* finished = nullptr;    // max_episode_steps > 0: dones | truncated of the last step [N] (k_truncate)
   int64_t exported;          // live DLPack exports
   std::string err;
 };
@@ -395,7 +397,7 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
       cfg->n_agents + cfg->n_boxes + cfg->n_heals > cfg->grid_size * cfg->grid_size ||
       cfg->inv_slots < 1 || cfg->inv_slots > MSV_MAX_SLOTS || cfg->zone_n_radiuses + 1 > MSV_MAX_ZONES ||
       cfg->zone_phases > cfg->zone_n_radiuses + 1 || cfg->lidar_n < 0 || cfg->lidar_n > MSV_MAX_LASERS ||
-      cfg->zone_phases < 1 || env_offset < 0 || env_offset + (int64_t)num_envs > (int64_t)1 << 32)   // Philox counter word 0 is 32 bits
+      cfg->zone_phases < 1 || cfg->max_episode_steps < 0 || env_offset < 0 || env_offset + (int64_t)num_envs > (int64_t)1 << 32)   // Philox counter word 0 is 32 bits
     return MSV_ERR_INVALID;
   {  // b2PolygonShape::Set welds vertices closer than its tolerance: a box that small is not a box any more (Box2D asserts);
      // the kernel treats every box analytically, so such configs are refused instead of simulated differently
@@ -467,6 +469,7 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
   rc |= dalloc(h, &S.obm, N); rc |= dalloc(h, &S.omask, AC * N);
   rc |= dalloc(h, &S.tq, N / (size_t)h->C.epb); rc |= dalloc(h, &S.tq_tail, 4);
   rc |= dalloc(h, &h->d_actions, N * A * 6);
+  if (cfg->max_episode_steps > 0) { rc |= dalloc(h, &h->truncated, N); rc |= dalloc(h, &h->finished, N); }
   rc |= dalloc(h, &h->d_stat_reward, (size_t)MSV_MAX_AGENTS); rc |= dalloc(h, &h->d_stat_kills, (size_t)MSV_MAX_AGENTS);
   rc |= dalloc(h, &h->d_stat_misc, (size_t)4);
   if (rc) { g_err = h->err; msv_destroy(h); return MSV_ERR_ALLOC; }
@@ -570,6 +573,7 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
   reg(h, "episode_length", O.episode_length, 2, {n});
   if (cfg->immunity_cooldown >= 0) reg(h, "immune", O.immune, 1, {n});
   if (cfg->battle_royale) { reg(h, "br_over", O.br_over, 1, {n}); reg(h, "br_results", O.br_results, 1, {n, a}); }
+  if (cfg->max_episode_steps > 0) reg(h, "truncated", h->truncated, 1, {n});
   if (cfg->auto_reset == 2) {   // same shapes, "terminal_" prefix
     std::map<std::string, TensorInfo> extra;
     static const char* names[MSV_OBS_KEYS] = {"agent", "others", "others_mask", "zone", "heals", "heals_mask", "heal_slot",
@@ -670,7 +674,8 @@ static void tmark(msv_handle* h, cudaStream_t st) {
   cudaEventRecord(h->tev[h->tev_used++], st);
 }
 
-static int launch(msv_handle* h, int which, const uint8_t* actions, void* stream) {
+// which: 0 step (dev_in = the actions), 1 reset (dev_in = the mask of the envs to reset, NULL = every env), 2 observe
+static int launch(msv_handle* h, int which, const uint8_t* dev_in, void* stream) {
   DevGuard g(h->device);
   cudaStream_t st = (cudaStream_t)stream;
   if (h->copy_pending) {                        // a read-back of the previous step may still be reading the arena
@@ -681,30 +686,51 @@ static int launch(msv_handle* h, int which, const uint8_t* actions, void* stream
   if (timed) tmark(h, st);
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
   const bool capturing = cudaStreamIsCapturing(st, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone;
+  // Terminal capture and the step limit split the step: k_step without the in-kernel reset, then the kernels that
+  // need the finished episodes' last state, then the reset of the finished environments.
+  const int T = h->cfg.max_episode_steps;
+  const bool split = which == 0 && (h->cfg.auto_reset == 2 || T > 0);
   // Tile hand-off (DevConst::tq_ticket): the observation kernel is launched programmatically dependent on the
   // step kernel and consumes the step kernel's blocks in the order they finish, so the observation of a finished
   // tile is written while the step's slow blocks (a wedged agent, a multi-agent island, a reset) still run.
-  // Needs the two launches adjacent in the stream: off under kernel timing, stream capture and terminal capture.
+  // Needs the two launches adjacent in the stream: off under kernel timing, stream capture and a split step.
   DevConst Cq = h->C;
-  const bool handoff = which == 0 && h->cfg.auto_reset != 2 && !timed && !capturing && h->handoff;
+  const bool handoff = which == 0 && !split && !timed && !capturing && h->handoff;
   if (handoff) {
     if (++h->tq_ticket == 0u) h->tq_ticket = 1u;
     Cq.tq_ticket = h->tq_ticket; Cq.tq_base = h->tq_base;
     Cq.pdl_wait = (h->step_pdl && h->last_was_step && h->last_stream == st) ? 1u : 0u;   // the previous call on this stream ended with this handle's observation kernels
     h->tq_base += (uint32_t)(h->C.N / h->C.epb);
   }
-  if (which == 0 && h->cfg.auto_reset == 2) {
-    // step without the in-kernel reset, keep the finished episodes' last observation, then
-    // reset exactly the envs that finished (same Philox streams as the in-kernel reset)
+  if (split) {
+    // step without the in-kernel reset; flag the episodes the step limit ends (finished = dones | truncated); keep
+    // the finished episodes' last observation; reset exactly the finished envs (same Philox streams as the in-kernel reset)
     DevConst C0 = h->C; C0.auto_reset = 0;
-    CK(msv_launch(h->cap, 0, C0, h->S, h->O, actions, st));
+    CK(msv_launch(h->cap, 0, C0, h->S, h->O, dev_in, st));
+    h->launches += 1;
     { int rc = readback(h, st); if (rc) return rc; }
-    CK(msv_launch_obs(h->C, h->S, h->obs_term, h->AC, h->O.dones, st));
-    if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O_term, h->BC, h->HC, st)); h->launches++; }
-    CK(msv_launch(h->cap, 4, h->C, h->S, h->O, nullptr, st));
-    h->launches += 3;
+    const uint8_t* fin = h->O.dones;
+    if (T > 0) {
+      CK(msv_launch_truncate(h->C, h->S, h->O, T, h->truncated, h->finished, st));
+      h->launches += 1;
+      fin = h->finished;
+    }
+    if (h->cfg.auto_reset == 2) {
+      CK(msv_launch_obs(h->C, h->S, h->obs_term, h->AC, fin, st));
+      h->launches += 1;
+      if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O_term, h->BC, h->HC, st)); h->launches++; }
+    }
+    if (h->cfg.auto_reset != 0) {
+      CK(msv_launch_reset(h->cap, h->C, h->S, h->O, fin, 1, nullptr, st));
+      h->launches += 1;
+    }
+  } else if (which == 1) {
+    // observations are a pure function of the state: the unmasked rows of a masked reset are rewritten with the
+    // values they already hold by the full observation pass below
+    CK(msv_launch_reset(h->cap, h->C, h->S, h->O, dev_in, 0, h->truncated, st));
+    h->launches += 1;
   } else {
-    CK(msv_launch(h->cap, which, Cq, h->S, h->O, actions, st));
+    CK(msv_launch(h->cap, which, Cq, h->S, h->O, dev_in, st));
     h->launches += 1;
     if (which == 0 && !handoff) { int rc = readback(h, st); if (rc) return rc; }
   }
@@ -781,6 +807,10 @@ int msv_debug_obs_kernel(msv_handle* h, void* stream) {
 }
 
 int msv_reset(msv_handle* h, void* stream) { return h ? launch(h, 1, nullptr, stream) : MSV_ERR_INVALID; }
+int msv_reset_envs(msv_handle* h, const uint8_t* mask_dev, void* stream) {
+  if (!h || !mask_dev) return MSV_ERR_INVALID;
+  return launch(h, 1, mask_dev, stream);
+}
 int msv_observe(msv_handle* h, void* stream) { return h ? launch(h, 2, nullptr, stream) : MSV_ERR_INVALID; }
 int msv_step(msv_handle* h, const uint8_t* actions_dev, void* stream) {
   if (!h || !actions_dev) return MSV_ERR_INVALID;
@@ -1149,7 +1179,7 @@ int64_t msv_obs_bytes_per_env(msv_handle* h) { return h ? (int64_t)h->obs.n_elem
 int64_t msv_kernel_launches(msv_handle* h) { return h ? h->launches : 0; }
 int msv_tile_plan(msv_handle* h, int32_t out[4]) {
   if (!h || !out) return MSV_ERR_INVALID;
-  out[0] = h->C.epb; out[1] = h->C.N / h->C.epb; out[2] = h->C.epb * h->AC; out[3] = (h->handoff && h->cfg.auto_reset != 2) ? 1 : 0;
+  out[0] = h->C.epb; out[1] = h->C.N / h->C.epb; out[2] = h->C.epb * h->AC; out[3] = (h->handoff && h->cfg.auto_reset != 2 && h->cfg.max_episode_steps == 0) ? 1 : 0;
   return MSV_OK;
 }
 

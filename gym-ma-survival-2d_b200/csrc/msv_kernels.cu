@@ -4,7 +4,8 @@
 //           of G lanes per environment (lane g = agent g, see msv_env.cuh):
 //           queue_actions -> pre_step hooks -> b2World::Step x2 -> post_step
 //           hooks -> observations -> rewards -> done -> stats (-> auto-reset).
-// k_reset : BaseEnv.reset (env:59-74) for every environment.
+// k_reset : BaseEnv.reset (env:59-74) for every environment, or for those a mask selects.
+// k_truncate: the step limit (truncated flags, finished mask) between k_step and the resets.
 // k_observe: fetch_observations only (after msv_set_state).
 // k_stats : flush_stats reduction.
 #include <cstdlib>
@@ -179,17 +180,24 @@ k_step(const __grid_constant__ DevConst C, const __grid_constant__ DevState S,
 #endif
 }
 
+// BaseEnv.reset (env:59-74) of the environments whose byte in `mask` is set (NULL: every environment).
+// finished != 0: the reset ends an episode that just finished (terminal capture, step limit): it is counted in
+// flush_stats()['episodes'], and the step's outputs (rewards, dones, episode_*) stay as the step wrote them.  The
+// masks of those resets (dones, k_truncate's finished mask) cover the padded batch.
+// finished == 0: a restart the caller asked for (msv_reset, msv_reset_envs): not counted, and the environment's
+// rewards, dones, truncated (when the handle has a step limit) and BattleRoyale flags are zeroed.  The caller's
+// mask has one byte per real environment.
 template <int AC, int BC, int HC, int G>
 __global__ void __launch_bounds__(MSV_TPB)
 k_reset(const __grid_constant__ DevConst C, const __grid_constant__ DevState S,
-        const __grid_constant__ DevOut Oc, int only_done) {
+        const __grid_constant__ DevOut Oc, const uint8_t* __restrict__ mask, int finished, uint8_t* __restrict__ truncated) {
   MSV_GROUP_SETUP(G);
   DevOut O = Oc;
-  if (only_done && !O.dones[e]) return;    // auto_reset = 2: only the envs that just finished (whole group leaves)
+  if (mask && ((!finished && e >= C.n_real) || !mask[e])) return;    // (whole group leaves)
   Env<AC, BC, HC, G> env(C, S, es, g, gmask, e);
   env.load();
   if (env.lead) {
-    if (only_done) env.LI(env.L_STEPISODES)++;
+    if (finished) env.LI(env.L_STEPISODES)++;
     MSV_COLD_ON(env, reset());
   }
   env.share_counts();
@@ -197,13 +205,33 @@ k_reset(const __grid_constant__ DevConst C, const __grid_constant__ DevState S,
   if (env.lead) {
     env.store_obm();
     env.store_immune(O);
-    if (!only_done) {
+    if (!finished) {
       for (int i = 0; i < C.A; ++i) O.rewards[(size_t)e * C.A + i] = 0.0f;
       O.dones[e] = 0;
+      if (truncated) truncated[e] = 0;
       if (C.battle_royale) { O.br_over[e] = 0; for (int i = 0; i < C.A; ++i) O.br_results[(size_t)e * C.A + i] = 0; }   // BattleRoyale.post_reset (sem:38-39)
     }
   }
   env.store();
+}
+
+// Step limit (msv_config.max_episode_steps = T > 0), after a k_step without the in-kernel reset: an episode that
+// has run T steps (hdr0.y) and did not end on this step is truncated.  Writes `truncated`, the episode_* rows of
+// the truncated environments (k_step wrote those of the finished ones) and `finished` = dones | truncated, the
+// rows the terminal capture keeps and the auto-reset resets.  One thread per environment of the padded batch.
+__global__ void __launch_bounds__(128)
+k_truncate(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, const __grid_constant__ DevOut O, int T,
+           uint8_t* __restrict__ truncated, uint8_t* __restrict__ finished) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= C.N) return;
+  const int steps = S.hdr0[e].y;
+  const bool done = O.dones[e] != 0, trunc = !done && steps >= T;
+  truncated[e] = trunc ? 1 : 0;
+  finished[e] = (done || trunc) ? 1 : 0;
+  if (trunc) {
+    for (int i = 0; i < C.A; ++i) O.episode_return[(size_t)e * C.A + i] = S.epret[i * C.N + e];
+    O.episode_length[e] = steps;
+  }
 }
 
 template <int AC, int BC, int HC, int G>
@@ -703,9 +731,15 @@ static cudaError_t launch_t(int which, const DevConst& C, const DevState& S, con
     return cudaLaunchKernelEx(&cfg, k_step<AC, BC, HC, G>, C, S, O, actions);
   }
   if (which == 0) k_step<AC, BC, HC, G><<<blocks, tpb, smem, st>>>(C, S, O, actions);
-  else if (which == 1) k_reset<AC, BC, HC, G><<<blocks, tpb, smem, st>>>(C, S, O, 0);
-  else if (which == 4) k_reset<AC, BC, HC, G><<<blocks, tpb, smem, st>>>(C, S, O, 1);
   else k_observe<AC, BC, HC, G><<<blocks, tpb, smem, st>>>(C, S, O);
+  return cudaPeekAtLastError();
+}
+
+template <int AC, int BC, int HC, int G>
+static cudaError_t reset_t(const DevConst& C, const DevState& S, const DevOut& O, const uint8_t* mask, int finished,
+                           uint8_t* truncated, cudaStream_t st) {
+  const size_t smem = (size_t)Env<AC, BC, HC, G>::SM_WORDS * C.epb * sizeof(float);
+  k_reset<AC, BC, HC, G><<<C.N / C.epb, C.epb * G, smem, st>>>(C, S, O, mask, finished, truncated);
   return cudaPeekAtLastError();
 }
 
@@ -716,6 +750,21 @@ cudaError_t msv_launch(int cap, int which, const DevConst& C, const DevState& S,
     case 1: return launch_t<4, 4, 4, 4>(which, C, S, O, actions, st);
     default: return launch_t<8, 8, 16, 8>(which, C, S, O, actions, st);
   }
+}
+
+cudaError_t msv_launch_reset(int cap, const DevConst& C, const DevState& S, const DevOut& O, const uint8_t* mask, int finished,
+                             uint8_t* truncated, cudaStream_t st) {
+  switch (cap) {
+    case 0: return reset_t<2, 4, 4, 2>(C, S, O, mask, finished, truncated, st);
+    case 1: return reset_t<4, 4, 4, 4>(C, S, O, mask, finished, truncated, st);
+    default: return reset_t<8, 8, 16, 8>(C, S, O, mask, finished, truncated, st);
+  }
+}
+
+cudaError_t msv_launch_truncate(const DevConst& C, const DevState& S, const DevOut& O, int T, uint8_t* truncated, uint8_t* finished,
+                                cudaStream_t st) {
+  k_truncate<<<(C.N + 127) / 128, 128, 0, st>>>(C, S, O, T, truncated, finished);
+  return cudaPeekAtLastError();
 }
 
 cudaError_t msv_launch_obs(const DevConst& C, const DevState& S, const ObsTable& T, int AC, const uint8_t* only_if, cudaStream_t st) {

@@ -5,9 +5,17 @@
 #ifndef MSV_TPB
 #define MSV_TPB 512   // maximum threads per block of k_step / k_reset / k_observe (the actual size is a runtime choice, see plan_blocks)
 #endif
-// cap: capacity class 0 = <2,4,4>, 1 = <4,4,4>, 2 = <8,8,16>; which: 0 step, 1 reset, 2 observe, 3 one-time kernel attribute setup, 4 reset only the envs whose done flag is set
+// cap: capacity class 0 = <2,4,4>, 1 = <4,4,4>, 2 = <8,8,16>; which: 0 step, 2 observe, 3 one-time kernel attribute setup
 cudaError_t msv_launch(int cap, int which, const DevConst& C, const DevState& S, const DevOut& O,
                        const uint8_t* actions, cudaStream_t st);
+// k_reset of the envs whose mask byte is set (mask NULL: every env).  finished != 0: the reset ends a finished
+// episode (counted, outputs kept; the mask covers the padded batch); 0: a restart (not counted, the env's rewards,
+// dones, truncated -- when not NULL -- and BattleRoyale flags are zeroed; the mask covers the real envs).
+cudaError_t msv_launch_reset(int cap, const DevConst& C, const DevState& S, const DevOut& O, const uint8_t* mask, int finished,
+                             uint8_t* truncated, cudaStream_t st);
+// k_truncate: step limit T > 0 after a step without the in-kernel reset; writes truncated and finished (uint8[N])
+cudaError_t msv_launch_truncate(const DevConst& C, const DevState& S, const DevOut& O, int T, uint8_t* truncated, uint8_t* finished,
+                                cudaStream_t st);
 void msv_capacity(int cap, int* AC, int* BC, int* HC, int* P, int* PW, int* sm_words);
 cudaError_t msv_launch_stats(int N, int stride, int AC, float* sreward, int* skills, int4* smisc, double* out_reward,
                              unsigned long long* out_kills, unsigned long long* out_misc, cudaStream_t st);

@@ -18,7 +18,7 @@ ERRORS = {-1: 'MSV_ERR_INVALID', -2: 'MSV_ERR_CUDA', -3: 'MSV_ERR_NO_DEVICE',
 
 EXPORTS = [
     'msv_abi_version', 'msv_sizeof_config', 'msv_sizeof_env_state', 'msv_sizeof_stats',
-    'msv_default_config', 'msv_create', 'msv_destroy', 'msv_reset', 'msv_step',
+    'msv_default_config', 'msv_create', 'msv_destroy', 'msv_reset', 'msv_reset_envs', 'msv_step',
     'msv_step_host', 'msv_step_host_obs', 'msv_step_host_async', 'msv_step_host_wait', 'msv_obs_host_bytes',
     'msv_obs_host_offset', 'msv_device_bytes', 'msv_tensor', 'msv_tensor_info', 'msv_get_state', 'msv_set_state',
     'msv_observe', 'msv_flush_stats', 'msv_bytes_per_env_step', 'msv_kernel_bytes_per_env', 'msv_obs_bytes_per_env', 'msv_kernel_launches', 'msv_tile_plan', 'msv_plan_tile',
@@ -67,6 +67,7 @@ def load():
     L.msv_create.argtypes = [vp, i32, i32, u64, i64, ctypes.POINTER(vp)]
     L.msv_destroy.argtypes = [vp]
     L.msv_reset.argtypes = [vp, vp]
+    L.msv_reset_envs.argtypes = [vp, vp, vp]
     L.msv_step.argtypes = [vp, vp, vp]
     L.msv_step_host.argtypes = [vp, vp, vp, vp, vp]
     L.msv_step_host_obs.argtypes = [vp, vp, vp, vp, vp, vp]
@@ -172,6 +173,10 @@ class Handle:
 
     def reset(self, stream=0):
         check(load().msv_reset(self.h, stream), self.h)
+
+    def reset_envs(self, mask_ptr, stream=0):
+        """msv_reset_envs: `mask_ptr` is a device pointer to uint8[num_envs] (the caller checks it)."""
+        check(load().msv_reset_envs(self.h, mask_ptr, stream), self.h)
 
     def observe(self, stream=0):
         check(load().msv_observe(self.h, stream), self.h)

@@ -108,8 +108,9 @@ def _radius(shape):
     return float(shape)
 
 
-def pack_config(cfg, continuous_melee=False, auto_reset=False):
-    """Nested (merged) config dict -> msv_config record (numpy void)."""
+def pack_config(cfg, continuous_melee=False, auto_reset=False, max_episode_steps=0):
+    """Nested (merged) config dict -> msv_config record (numpy void).  `max_episode_steps`: the
+    step limit of the vector env (0 = none), an extension the reference does not have."""
     rec = np.zeros((), dtype=CONFIG_DT)
     agents = cfg['agents']
     rec['n_agents'] = agents.get('n_spawns', agents.get('n_agents'))
@@ -181,6 +182,7 @@ def pack_config(cfg, continuous_melee=False, auto_reset=False):
     rec['b2_variant'] = int(cfg.get('box2d', {}).get('variant', 0))
     # False/0 off, True/1 in-kernel reset, 'terminal'/2 reset + terminal observation capture
     rec['auto_reset'] = 2 if auto_reset in ('terminal', 2) else int(bool(auto_reset))
+    rec['max_episode_steps'] = int(max_episode_steps)
     validate(rec)
     return rec
 
@@ -205,6 +207,8 @@ def validate(rec):
         raise ValueError('too many safe-zone radiuses')
     if int(rec['lidar_n']) > D['MSV_MAX_LASERS']:
         raise ValueError(f'lidars.n_lasers must be <= {D["MSV_MAX_LASERS"]}')
+    if int(rec['max_episode_steps']) < 0:
+        raise ValueError('max_episode_steps must be >= 0 (0: no step limit)')
     if rec['teams'] and A < 2:
         raise ValueError('teams need at least 2 agents')
 

@@ -36,13 +36,21 @@ class MaSurvivalVec:
                             lidar_frac / lidar_hit included when lidars are
                             configured (one more lidar scan per step, in this
                             mode only)
+    max_episode_steps : int|None  step limit (vector-env extension; None or 0:
+                            none).  An episode that has run this many steps
+                            without ending on the last one is truncated:
+                            step()'s info['truncated'] flags it, episode_return /
+                            episode_length rows are valid where done | truncated,
+                            and auto_reset treats it like a finished episode
+                            (auto_reset=False only flags it: see reset_envs)
     """
 
     metadata = {'render_modes': ['rgb_array'], 'render_fps': 30}
 
-    def __init__(self, config=None, num_envs=1, device=0, seed=0, env_offset=0, auto_reset=True):
+    def __init__(self, config=None, num_envs=1, device=0, seed=0, env_offset=0, auto_reset=True, max_episode_steps=None):
         self.config, self._continuous_melee = merge_config(config)
-        self._rec = pack_config(self.config, self._continuous_melee, auto_reset=auto_reset)
+        self._rec = pack_config(self.config, self._continuous_melee, auto_reset=auto_reset,
+                                max_episode_steps=max_episode_steps or 0)
         self.num_envs = int(num_envs)
         self.device = int(device)
         self.auto_reset = bool(auto_reset)
@@ -53,7 +61,9 @@ class MaSurvivalVec:
         self.steps = 0
         self._act_buf = None
         self._done_bool = None
+        self._trunc_bool = None
         self._host_obs = None
+        self._mask_buf = None
 
     # ---- reference properties (env:245-291) --------------------------------
     @property
@@ -127,11 +137,50 @@ class MaSurvivalVec:
 
     def reset(self, seed=None, return_info=False, options=None):
         """BaseEnv.reset (env:59-74) for all N envs (the `seed` argument is
-        ignored, as in the reference)."""
+        ignored, as in the reference).  options={'reset_mask': m} resets only
+        the envs `m` selects (see reset_envs)."""
+        if options and 'reset_mask' in options:
+            obs = self.reset_envs(options['reset_mask'])
+            return (obs, {}) if return_info else obs
         self._h.reset(self._stream())
         self.steps = 0
         obs = self._obs()
         return (obs, {}) if return_info else obs
+
+    def reset_envs(self, mask):
+        """BaseEnv.reset (env:59-74) for the chosen envs only; the others are left untouched.  `mask`: a
+        CUDA bool or uint8 tensor of N elements on this device (used in place, no host synchronisation: a
+        step and a reset_envs can be captured together in a CUDA graph), a host boolean array of N, or a
+        sequence of env indices.  A reset env starts its next episode (the draws an auto-reset would make);
+        its rewards, dones and truncated flags are zeroed; its episode_return / episode_length rows, which
+        describe the last finished episode, are kept, and flush_stats() does not count the interrupted
+        episode.  Returns the observation dict."""
+        import torch
+        N, dev = self.num_envs, f'cuda:{self.device}'
+        if isinstance(mask, torch.Tensor) and mask.is_cuda:
+            if mask.device.index != self.device:
+                raise ValueError(f'reset mask lives on {mask.device}, the environments on {dev}')
+            if mask.dtype not in (torch.bool, torch.uint8) or mask.numel() != N:
+                raise ValueError(f'a device reset mask must be a bool or uint8 tensor of {N} elements')
+            m = mask.reshape(N).contiguous()
+        else:
+            arr = np.asarray(mask.cpu() if isinstance(mask, torch.Tensor) else mask)
+            if arr.dtype == np.bool_:
+                if arr.size != N:
+                    raise ValueError(f'a host reset mask must have {N} elements')
+                m = arr.reshape(N)
+            elif arr.size == 0 or np.issubdtype(arr.dtype, np.integer):
+                idx = arr.reshape(-1).astype(np.int64)
+                if ((idx < 0) | (idx >= N)).any():
+                    raise ValueError(f'env indices must be in 0..{N - 1}')
+                m = np.zeros(N, dtype=np.bool_)
+                m[idx] = True
+            else:
+                raise ValueError('reset mask: a bool/uint8 CUDA tensor, a host boolean array or a sequence of env indices')
+            m = torch.from_numpy(np.ascontiguousarray(m)).to(dev)
+        self._mask_buf = m     # keep alive until the stream has consumed it
+        self._h.reset_envs(m.data_ptr(), self._stream())
+        return self._obs()
 
     def step(self, actions):
         """BaseEnv.step (env:76-90).  `actions`: integer array-like
@@ -157,9 +206,15 @@ class MaSurvivalVec:
         self._h.step(a.data_ptr(), self._stream())
         self.steps += 1
         info = {'terminal_observation': self._obs('terminal_')} if self._terminal else {}
-        # per-env episode statistics (rows valid where done): what a trainer logs at episode end
+        # per-env episode statistics (rows valid where done, or done | truncated under a step limit): what a
+        # trainer logs at episode end
         info['episode_return'] = self._h.tensor('episode_return')
         info['episode_length'] = self._h.tensor('episode_length')
+        if self._rec['max_episode_steps'] > 0:
+            trunc = self._h.tensor('truncated')
+            if self._trunc_bool is None or self._trunc_bool.data_ptr() != trunc.data_ptr():
+                self._trunc_bool = trunc.view(torch.bool)
+            info['truncated'] = self._trunc_bool
         for k in ('immune', 'br_over', 'br_results'):
             if self._h.has_tensor(k):
                 info[k] = self._h.tensor(k)

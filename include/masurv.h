@@ -117,7 +117,12 @@ typedef struct msv_config {
    * v *= 1/(1 + h*d); bit 1 = b2PolygonShape::Set weld tolerance (0.5*linearSlop)^2 instead of
    * 2.3.0's 0.5*linearSlop; bit 2 = SolveTOI gives up at toiCount >= b2_maxSubSteps instead of >. */
   int32_t b2_variant;
-  int32_t reserved0;
+  /* Vector-env extension (the reference has no step limit): 0 = none; T > 0 ends an episode as
+   * "truncated" once it has run T steps (msv_env_state.steps >= T) without ending on that step.
+   * Adds the "truncated" tensor (uint8[num_envs]); auto_reset resets truncated envs like finished ones
+   * (and auto_reset 2 keeps their last observation), auto_reset 0 only flags them (msv_reset_envs).
+   * The observation hand-off is off (msv_tile_plan out[3] = 0).  Negative values are refused. */
+  int32_t max_episode_steps;
 } msv_config;
 #define MSV_B2_CLAMP_DAMPING 1
 #define MSV_B2_WELD_SQUARED 2
@@ -247,6 +252,15 @@ int msv_destroy(msv_handle* h);
 /* Replaces BaseEnv.reset (env:59-74) for every env; stream-ordered. */
 int msv_reset(msv_handle* h, void* cuda_stream);
 
+/* Reset the environments whose byte in mask_dev (device pointer, uint8[num_envs], nonzero = reset)
+ * is set, as BaseEnv.reset (env:59-74) for each of them; stream-ordered.  A reset env starts its next
+ * episode (the same Philox draws as an auto-reset), gets msv_reset's observation, and its rewards,
+ * dones and truncated are zeroed; its episode_return / episode_length rows (the last FINISHED
+ * episode) stay, and the interrupted episode is not counted in msv_stats.episodes.  Every other env's
+ * state and outputs are left bit-identical.  No host synchronisation and no allocation: a step and a
+ * reset_envs can be captured together in a CUDA graph. */
+int msv_reset_envs(msv_handle* h, const uint8_t* mask_dev, void* cuda_stream);
+
 /* Replaces BaseEnv.step (env:76-90).  actions_dev: device pointer,
  * uint8[num_envs][n_agents][6], MultiDiscrete([3,3,3,2,2,2]) (env:451).
  * Results land in the library-owned tensors (msv_tensor). */
@@ -291,7 +305,11 @@ int64_t msv_obs_host_offset(msv_handle* h, const char* name); /* -1: unknown */
 
 /* Zero-copy export of a library-owned device tensor as DLPack.  Names are the
  * reference's observation keys (env:391-447) plus "rewards", "dones",
- * "lidar_frac", "lidar_kind".  The deleter only drops a refcount. */
+ * "episode_return", "episode_length", "lidar_frac", "lidar_hit", and
+ * "truncated" (uint8[num_envs], only with max_episode_steps > 0: 1 where the
+ * step limit ended the episode on the last step and the game did not; the
+ * episode_* rows are valid where dones | truncated).  The deleter only drops
+ * a refcount. */
 int msv_tensor(msv_handle* h, const char* name, struct DLManagedTensor** out);
 
 /* Raw view of the same tensors (for non-DLPack callers / tests). */
@@ -341,7 +359,8 @@ int64_t msv_kernel_launches(msv_handle* h); /* launches since create */
 /* How the batch is tiled onto the GPU: out[0] environments per thread block of
  * the step kernel, out[1] its blocks, out[2] its threads per block, out[3] 1 when
  * the observation kernels are launched programmatically dependent on the step
- * kernel and consume its tiles as they finish (the vectorised counterpart of
+ * kernel and consume its tiles as they finish (not with auto_reset 2 or a step
+ * limit, whose steps run more kernels in between; the vectorised counterpart of
  * env:76-90 has no analogue in the reference: it steps one env at a time). */
 int msv_tile_plan(msv_handle* h, int32_t out[4]);
 /* The planner behind it, without a device (pure host logic): how num_envs
