@@ -10,7 +10,6 @@
 #include <string>
 #include <vector>
 #include <map>
-#include <algorithm>
 
 #include "../../include/masurv.h"
 #include "msv_launch.h"
@@ -63,6 +62,7 @@ struct msv_handle {
   double* d_stat_reward; unsigned long long* d_stat_kills; unsigned long long* d_stat_misc;
   int64_t launches;
   ObsTable obs;
+  int64_t obs_floats = 0;    // floats of one environment's observation keys (the keys the config has)
   ObsTable obs_term;         // auto_reset == 2: same table, writing the "terminal_<key>" tensors
   DevOut O_term;             // auto_reset == 2: O with the lidar pointers on the "terminal_lidar_*" tensors
   uint8_t* truncated = nullptr;   // max_episode_steps > 0: the "truncated" tensor [N]
@@ -479,64 +479,14 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
     std::vector<int> se(N, INT32_MIN);              // no reset record drawn yet
     cudaMemcpy(S.spare_ep, se.data(), N * sizeof(int), cudaMemcpyHostToDevice);
   }
-  {  // observation element table for k_obs (env:391-447 shapes, env:510-657 contents)
-    std::vector<ObsDesc> D;
+  {  // the observation keys of k_obs2 (env:391-447 shapes)
     const int Ai = (int)A, Bi = (int)B, Hi = (int)H, Si = (int)Sw;
-    auto add = [&](int key, int off, int src, int slot, int comp, int aux) {
-      ObsDesc d; d.src = (uint8_t)src; d.slot = (uint8_t)slot; d.comp = (uint8_t)comp; d.aux = (uint8_t)aux;
-      d.key = (uint16_t)key; d.off = (uint16_t)off; D.push_back(d);
-    };
-    auto agent_row = [&](int key, int off, int i) {
-      int o = off;
-      add(key, o++, OS_AGENT_ID, i, 0, 0);
-      if (cfg->teams) add(key, o++, OS_AGENT_TEAM, i, 0, i < Ai / 2 ? 0 : 1);
-      add(key, o++, OS_AGENT_HEALTH, i, 0, 0);
-      add(key, o++, OS_AKIN0, i, 0, 0); add(key, o++, OS_AKIN0, i, 1, 0); add(key, o++, OS_AKIN0, i, 2, 0);
-      add(key, o++, OS_AKIN0, i, 3, 0); add(key, o++, OS_AKIN1, i, 0, 0); add(key, o++, OS_AKIN1, i, 1, 0);
-    };
     ObsKey* K = h->obs.keys;
     K[0] = {O.agent, Ai * Si}; K[1] = {O.others, Ai * (Ai - 1) * Si}; K[2] = {O.others_mask, Ai * (Ai - 1)}; K[3] = {O.zone, 6};
     K[4] = {O.heals, Hi * 2}; K[5] = {O.heals_mask, Ai * Hi}; K[6] = {O.heal_slot, Ai}; K[7] = {O.heal_slot_mask, Ai};
     K[8] = {O.boxes, Bi * 11}; K[9] = {O.boxes_mask, Ai * Bi}; K[10] = {O.box_items, Bi * 10}; K[11] = {O.box_items_mask, Ai * Bi};
     K[12] = {O.box_slot, Ai * 8}; K[13] = {O.box_slot_mask, Ai};
-    for (int i = 0; i < Ai; ++i) agent_row(0, i * Si, i);
-    for (int i = 0; i < Ai; ++i) { int k = 0; for (int j = 0; j < Ai; ++j) { if (j == i) continue; agent_row(1, (i * (Ai - 1) + k) * Si, j); add(2, i * (Ai - 1) + k, OS_OTHERS_MASK, i, j, 0); k++; } }
-    for (int c2 = 0; c2 < 3; ++c2) { add(3, c2, OS_ZONE_CUR, 0, c2, 0); add(3, 3 + c2, OS_ZONE_NEXT, 0, c2, 0); }
-    if (Hi > 0) {
-      for (int k = 0; k < Hi; ++k) { add(4, 2 * k, OS_HEAL, k, 0, 0); add(4, 2 * k + 1, OS_HEAL, k, 1, 0); }
-      for (int i = 0; i < Ai; ++i) { for (int k = 0; k < Hi; ++k) add(5, i * Hi + k, OS_LIST_MASK, k, i, 2); add(6, i, OS_HEAL_SLOT, i, 0, 0); add(7, i, OS_HEAL_SLOT_MASK, i, 0, 0); }
-    }
-    if (Bi > 0) {
-      for (int k = 0; k < Bi; ++k) {
-        for (int c2 = 0; c2 < 8; ++c2) { add(8, k * 11 + c2, OS_BOX_VERT, k, c2, 0); add(10, k * 10 + c2, OS_ITEM_VERT, k, c2, 0); }
-        for (int c2 = 0; c2 < 3; ++c2) add(8, k * 11 + 8 + c2, OS_BOX_POS, k, c2, 0);
-        for (int c2 = 0; c2 < 2; ++c2) add(10, k * 10 + 8 + c2, OS_ITEM_POS, k, c2, 0);
-      }
-      for (int i = 0; i < Ai; ++i) {
-        for (int k = 0; k < Bi; ++k) { add(9, i * Bi + k, OS_LIST_MASK, k, i, 0); add(11, i * Bi + k, OS_LIST_MASK, k, i, 1); }
-        for (int c2 = 0; c2 < 8; ++c2) add(12, i * 8 + c2, OS_BOX_SLOT, i, c2, 0);
-        add(13, i, OS_BOX_SLOT_MASK, i, 0, 0);
-      }
-    }
-    // group the table by key so that consecutive threads write consecutive floats
-    std::stable_sort(D.begin(), D.end(), [](const ObsDesc& x, const ObsDesc& y) { return x.key != y.key ? x.key < y.key : x.off < y.off; });
-    ObsDesc* dd = nullptr;
-    if (dalloc(h, &dd, D.size())) { g_err = h->err; msv_destroy(h); return MSV_ERR_ALLOC; }
-    cudaMemcpy(dd, D.data(), D.size() * sizeof(ObsDesc), cudaMemcpyHostToDevice);
-    h->obs.desc = dd; h->obs.n_elems = (int)D.size();
-    {  // compute order: grouped by source kind (then slot, component) so that the lanes of a warp take the same branch
-      std::vector<ObsDesc> Cd(D);
-      for (size_t i = 0; i < Cd.size(); ++i) { Cd[i].key = (uint16_t)i; Cd[i].off = 0; }
-      std::stable_sort(Cd.begin(), Cd.end(), [](const ObsDesc& x, const ObsDesc& y) {
-        if (x.src != y.src) return x.src < y.src;
-        if (x.aux != y.aux) return x.aux < y.aux;
-        if (x.slot != y.slot) return x.slot < y.slot;   // same slot adjacent: the lanes share the 16-byte state word
-        return x.comp < y.comp; });
-      ObsDesc* cd = nullptr;
-      if (dalloc(h, &cd, Cd.size())) { g_err = h->err; msv_destroy(h); return MSV_ERR_ALLOC; }
-      cudaMemcpy(cd, Cd.data(), Cd.size() * sizeof(ObsDesc), cudaMemcpyHostToDevice);
-      h->obs.cdesc = cd;
-    }
+    for (int k = 0; k < MSV_OBS_KEYS; ++k) if (obs_key_used(k, Hi, Bi)) h->obs_floats += K[k].chunk;
     h->obs_term = h->obs;
     if (cfg->auto_reset == 2) {
       for (int k = 0; k < MSV_OBS_KEYS; ++k) {
@@ -918,7 +868,7 @@ int64_t msv_device_bytes(msv_handle* h) { return h ? (int64_t)h->device_bytes : 
 
 /* debug/bench: CUDA-event timing of the kernels msv_step launches.  enable=1 starts recording (one
  * event pair per kernel and step, up to 8192 steps); enable=0 stops, synchronises and returns the
- * mean milliseconds of [k_step (+ terminal capture), k_obs, k_lidar] and the number of steps. */
+ * mean milliseconds of [k_step (+ terminal capture), k_obs2, k_lidar] and the number of steps. */
 int msv_debug_kernel_timing(msv_handle* h, int enable, double out_ms[3], int64_t* n_steps) {
   if (!h) return MSV_ERR_INVALID;
   DevGuard g(h->device);
@@ -1168,14 +1118,14 @@ int64_t msv_kernel_bytes_per_env(msv_handle* h, int32_t which) {
     const int64_t wr = 76 * A + 32 + 32 + 24 * PW + 16 + 8 + om + 4 * A + 1;
     return rd + wr;
   }
-  if (which == 1) return 48 * A + 8 + om + 16 + 32 * B + 16 * B + 8 * H + 40 + (int64_t)h->obs.n_elems * 4;
+  if (which == 1) return 48 * A + 8 + om + 16 + 32 * B + 16 * B + 8 * H + 40 + h->obs_floats * 4;
   if (which == 2) return L > 0 ? 16 + 32 * B + 16 * B + 8 * H + 32 * A + 8 * A * L : 0;
   return 0;
 }
 int64_t msv_bytes_per_env_step(msv_handle* h) {
   return msv_kernel_bytes_per_env(h, 0) + msv_kernel_bytes_per_env(h, 1) + msv_kernel_bytes_per_env(h, 2);
 }
-int64_t msv_obs_bytes_per_env(msv_handle* h) { return h ? (int64_t)h->obs.n_elems * 4 : 0; }
+int64_t msv_obs_bytes_per_env(msv_handle* h) { return h ? h->obs_floats * 4 : 0; }
 int64_t msv_kernel_launches(msv_handle* h) { return h ? h->launches : 0; }
 int msv_tile_plan(msv_handle* h, int32_t out[4]) {
   if (!h || !out) return MSV_ERR_INVALID;

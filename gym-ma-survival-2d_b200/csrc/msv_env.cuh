@@ -2140,7 +2140,7 @@ struct Env {
   // ======================================================================
   // others_mask (env:692-703) as bits: bit (i*AC + j) set <=> observer i sees
   // agent j.  Q1: Cameras.seen is looked up by the POST-death list position.
-  // The observation tensors themselves are written by k_obs (msv_kernels.cu).
+  // The observation tensors themselves are written by k_obs2 (msv_kernels.cu).
   // [leader]
   DEV void store_obm() {
     unsigned long long bits = 0ull;

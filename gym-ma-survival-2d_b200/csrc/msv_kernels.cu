@@ -151,7 +151,7 @@ k_step(const __grid_constant__ DevConst C, const __grid_constant__ DevState S,
   }
   PROF(9);
   PHASE_SYNC(8);
-  if (env.lead) env.store_obm();           // env:84: the observation tensors are gathered by k_obs
+  if (env.lead) env.store_obm();           // env:84: the observation tensors are gathered by k_obs2
   PROF(10);
   env.store();
   PROF(11);
@@ -245,113 +245,20 @@ k_observe(const __grid_constant__ DevConst C, const __grid_constant__ DevState S
   if (env.lead) env.store_obm();
 }
 
-// fetch_observations (env:510-657): one thread per output float, gathered from
-// the SoA state after k_step / k_reset / k_observe stored it.  A block covers
-// OBS_EPB consecutive environments (evaluated in source-kind order into shared memory, then
-// written in output order): a thread reads its element descriptor once
-// and emits that element for each of them (their SoA words share sectors);
-// consecutive threads write consecutive floats of a key -> coalesced stores.
-// value of one observation element of environment e (see ObsDesc)
-__device__ __forceinline__ float obs_value(const DevConst& C, const DevState& S, const ObsDesc d, int e, int AC) {
-  const int N = C.N;
-  float v = 0.0f;
-  auto alive = [&](int i) { return (__float_as_int(S.akin1[i * N + e].w) & 1) != 0; };
-  auto vert = [&](float hx, float hy, int rot, int comp) {   // b2PolygonShape vertex order (Q8)
-    int j = ((comp >> 1) + rot) & 3;
-    return (comp & 1) ? ((j >= 2) ? hy : -hy) : ((j == 1 || j == 2) ? hx : -hx);
-  };
-  switch (d.src) {
-    case OS_AGENT_ID: v = (float)d.slot; break;
-    case OS_AGENT_TEAM: v = (float)d.aux; break;
-    case OS_AGENT_HEALTH: if (alive(d.slot)) v = (float)S.aint[d.slot * N + e].x; break;
-    case OS_AKIN0: if (alive(d.slot)) { float4 k = S.akin0[d.slot * N + e]; v = d.comp == 0 ? k.x : d.comp == 1 ? k.y : d.comp == 2 ? k.z : k.w; } break;
-    case OS_AKIN1: if (alive(d.slot)) { float4 k = S.akin1[d.slot * N + e]; v = d.comp == 0 ? k.x : k.y; } break;
-    case OS_OTHERS_MASK: v = ((S.obm[e] >> (d.slot * AC + d.comp)) & 1ull) ? 0.0f : 1.0f; break;
-    case OS_ZONE_CUR: { float4 z = S.zonecur[e]; v = d.comp == 0 ? z.x : d.comp == 1 ? z.y : z.z; } break;
-    case OS_ZONE_NEXT: {
-      int ph = S.zoneint[e].x;
-      if (ph < C.zone_phases - 1) {
-        if (d.comp == 2) v = C.zone_r32[ph + 1];
-        else { float2 c = S.zonec[(ph + 1) * N + e]; v = d.comp == 0 ? c.x : c.y; }
-      }
-    } break;
-    case OS_HEAL: { int nh = (S.hdr0[e].x >> 16) & 255; if (d.slot < nh) { float2 h = S.heal[d.slot * N + e]; v = d.comp == 0 ? h.x : h.y; } } break;
-    case OS_LIST_MASK: {   // aux: 0 boxes, 1 box items, 2 heals; comp = observer
-      int cnt = (S.hdr0[e].x >> (d.aux * 8)) & 255;
-      if (C.omniscient) v = d.slot < cnt ? 0.0f : 1.0f;                      // env:564-568
-      else {                                                                  // env:706-739
-        int bitpos = d.aux == 2 ? d.slot : (d.aux == 0 ? 16 + d.slot : 24 + d.slot);
-        bool seen = d.slot < cnt && alive(d.comp) && ((S.omask[d.comp * N + e] >> bitpos) & 1u);
-        v = seen ? 0.0f : 1.0f;
-      }
-    } break;
-    case OS_HEAL_SLOT: case OS_HEAL_SLOT_MASK: case OS_BOX_SLOT: case OS_BOX_SLOT_MASK: {
-      int want = (d.src == OS_HEAL_SLOT || d.src == OS_HEAL_SLOT_MASK) ? MSV_ITEM_HEAL : MSV_ITEM_BOX;
-      int inv = S.aint[d.slot * N + e].w, n = inv & 7;
-      bool has = alive(d.slot) && n > 0 && ((inv >> (4 + 2 * (n - 1))) & 3) == want;
-      if (d.src == OS_HEAL_SLOT) v = has ? (float)C.healing : 0.0f;
-      else if (d.src == OS_HEAL_SLOT_MASK || d.src == OS_BOX_SLOT_MASK) v = has ? 0.0f : 1.0f;
-      else if (has) { float4 pl = S.ainv[(d.slot * 4 + n - 1) * N + e]; v = vert(pl.x, pl.y, __float_as_int(pl.w) & 1, d.comp); }
-    } break;
-    case OS_BOX_VERT: case OS_BOX_POS: {
-      int nb = S.hdr0[e].x & 255;
-      if (d.slot < nb) {
-        float4 b0 = S.box0[d.slot * N + e];
-        if (d.src == OS_BOX_POS) v = d.comp == 0 ? b0.x : d.comp == 1 ? b0.y : 0.0f;
-        else v = vert(b0.z, b0.w, (S.box1[d.slot * N + e].y >> 1) & 1, d.comp);
-      }
-    } break;
-    case OS_ITEM_VERT: case OS_ITEM_POS: {
-      int ni = (S.hdr0[e].x >> 8) & 255;
-      if (d.slot < ni) {
-        float4 it = S.item0[d.slot * N + e];
-        if (d.src == OS_ITEM_POS) v = d.comp == 0 ? it.x : it.y;
-        else v = vert(it.z, it.w, 1, d.comp);
-      }
-    } break;
-    default: break;
-  }
-  return v;
-}
-
-#define OBS_EPB 4   // environments per block (measured: 1 -> 32.9, 2 -> 28.8, 4 -> 28.2, 8 -> 34.2, 16 -> 48.3 us for 16 384 envs of 2v2)
-__global__ void __launch_bounds__(256)
-k_obs(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, const __grid_constant__ ObsTable Tb, int AC,
-      const uint8_t* __restrict__ only_if) {
-  extern __shared__ float stage[];           // [OBS_EPB][n_elems] values in output order
-  const int e0 = blockIdx.x * OBS_EPB, n = Tb.n_elems;
-  bool on[OBS_EPB];
-#pragma unroll
-  for (int j = 0; j < OBS_EPB; ++j) { const int e = e0 + j; on[j] = e < C.n_real && (!only_if || only_if[e]); }
-  // phase 1: evaluate the elements in source-kind order (the lanes of a warp take the same branch)
-  for (int t = threadIdx.x; t < n; t += 256) {
-    const ObsDesc d = Tb.cdesc[t];           // read once, reused for the block's environments
-#pragma unroll
-    for (int j = 0; j < OBS_EPB; ++j) stage[j * n + d.key] = on[j] ? obs_value(C, S, d, e0 + j, AC) : 0.0f;
-  }
-  __syncthreads();
-  // phase 2: write them out in output order: consecutive threads, consecutive floats of a key
-  for (int el = threadIdx.x; el < n; el += 256) {
-    const ObsDesc d = Tb.desc[el];
-    const ObsKey k = Tb.keys[d.key];
-#pragma unroll
-    for (int j = 0; j < OBS_EPB; ++j)
-      if (on[j]) k.base[(size_t)(e0 + j) * k.chunk + d.off] = stage[j * n + el];
-  }
-}
-
-
-// fetch_observations, fast path (every environment, no row filter).  The descriptor-driven kernel
-// above evaluates one output float per thread (~100 instructions each); this one works SOURCE-major:
-// a warp takes one source item -- agent j, box k, floor item k, heal k, the zone -- for 32
-// consecutive environments (lane = environment: the SoA loads are fully coalesced), builds
-// everything that item contributes (an agent row goes to `agent` and to the `others` block of every
-// other observer; observer j's mask rows and inventory-slot views) and scatters it into a
-// shared-memory stage laid out exactly like the 32-environment slice of each output tensor.  The
-// stage is then copied out with 16-byte stores, one contiguous run per tensor.
+// fetch_observations (env:510-657), SOURCE-major: a warp takes one source item -- agent j, box k,
+// floor item k, heal k, the zone -- for 32 consecutive environments (lane = environment: the SoA
+// loads are fully coalesced), builds everything that item contributes (an agent row goes to `agent`
+// and to the `others` block of every other observer; observer j's mask rows and inventory-slot views)
+// and scatters it into a shared-memory stage laid out exactly like the 32-environment slice of each
+// output tensor.  The stage is then copied out with 16-byte stores, one contiguous run per tensor.
+// kRows (terminal capture): only the rows of real environments whose `only_if` byte is set are
+// written, with scalar stores (a row's slice of a key is not 16-byte aligned in general); the other
+// rows of the output are left untouched, and a tile without such a row leaves at once.
 #define OBS2_E 32
+template <bool kRows>
 __global__ void __launch_bounds__(1024)
-k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, const __grid_constant__ ObsTable Tb, int AC) {
+k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, const __grid_constant__ ObsTable Tb, int AC,
+       const uint8_t* __restrict__ only_if) {
   extern __shared__ float stage[];
   const int A = C.A, B = C.B0, H = C.H0, Sw = C.S, N = C.N;
   // A tile is (part of) the environments of one k_step block: block `kb`, sub-tile `sub` of up to OBS2_E rows.
@@ -361,7 +268,7 @@ k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, c
   int kb = blockIdx.x / spb; const int sub = blockIdx.x - kb * spb;
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   TRACE(2, blockIdx.x);
-  if (C.tq_ticket) {
+  if (!kRows && C.tq_ticket) {                   // (a row-filtered launch is never part of a hand-off)
     __shared__ int s_kb;
     if (threadIdx.x == 0) {
       const unsigned long long* q = S.tq + kb;
@@ -396,6 +303,11 @@ k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, c
   }
   const int e = e0 + lane;
   const bool live = lane < rows;                 // (e < N: the padded batch is a whole number of k_step blocks)
+  unsigned sel = 0u;                             // kRows: bit r = row r is written (every warp computes the same mask)
+  if (kRows) {
+    sel = __ballot_sync(0xffffffffu, live && e < C.n_real && only_if[e] != 0);
+    if (!sel) return;
+  }
   const int n_items = A + 2 * B + H + 1;
   // (state loads below bypass L1 -- __ldcg: each word is read once, and with the hand-off on it was written by a
   // block of the still-running step kernel on another SM)
@@ -487,14 +399,21 @@ k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, c
   TRACE(5, blockIdx.x);
   for (int k = 0; k < MSV_OBS_KEYS; ++k) {
     const int chunk = Tb.keys[k].chunk;
-    if (chunk <= 0 || (k >= 4 && k <= 7 && H == 0) || (k >= 8 && B == 0)) continue;   // key groups the config does not have
-    const int n4 = rows * chunk / 4;
-    const float4* src = reinterpret_cast<const float4*>(stage + koff[k]);
-    float4* dst = reinterpret_cast<float4*>(Tb.keys[k].base + (size_t)e0 * chunk);
-    for (int q = threadIdx.x; q < n4; q += blockDim.x) dst[q] = src[q];
+    if (chunk <= 0 || !obs_key_used(k, H, B)) continue;
+    if (kRows) {
+      const float* src = stage + koff[k];
+      float* dst = Tb.keys[k].base + (size_t)e0 * chunk;
+      for (int q = threadIdx.x; q < rows * chunk; q += blockDim.x)
+        if ((sel >> (q / chunk)) & 1u) dst[q] = src[q];
+    } else {
+      const int n4 = rows * chunk / 4;
+      const float4* src = reinterpret_cast<const float4*>(stage + koff[k]);
+      float4* dst = reinterpret_cast<float4*>(Tb.keys[k].base + (size_t)e0 * chunk);
+      for (int q = threadIdx.x; q < n4; q += blockDim.x) dst[q] = src[q];
+    }
   }
   TRACE(4, blockIdx.x);
-  if (C.tq_ticket) {
+  if (!kRows && C.tq_ticket) {
     // The last tile to finish waits for the step kernel's grid to have completed, so that "this grid is complete"
     // implies "the step kernel is complete" for whatever follows in the stream, whichever way the runtime orders
     // a third kernel after a programmatic pair.  (Every other block has already seen its tile's release.)
@@ -707,6 +626,17 @@ __global__ void k_stats(int N, int stride, int AC, float* sreward, int* skills, 
 }
 
 // ------------------------------------------------------------- launchers ---
+template <bool kRows>
+static cudaError_t obs_attrs() {
+  // the stage of the 8-agent class is ~1 000 floats x 32 environments, far over the 48 KB default
+  cudaError_t e = cudaFuncSetAttribute(k_obs2<kRows>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  // same L1/shared split as the step kernel, so that a tile can become resident on an SM that still runs one of its blocks
+  const char* cv = getenv("MSV_OBS_CARVEOUT");
+  if (e == cudaSuccess && (!cv || atoi(cv) != 0))
+    e = cudaFuncSetAttribute(k_obs2<kRows>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  return e;
+}
+
 template <int AC, int BC, int HC, int G>
 static cudaError_t launch_t(int which, const DevConst& C, const DevState& S, const DevOut& O,
                             const uint8_t* actions, cudaStream_t st) {
@@ -715,10 +645,12 @@ static cudaError_t launch_t(int which, const DevConst& C, const DevState& S, con
   size_t smem = (size_t)Env<AC, BC, HC, G>::SM_WORDS * epb * sizeof(float);
   size_t smem_max = (size_t)Env<AC, BC, HC, G>::SM_WORDS * (MSV_TPB / G) * sizeof(float);
   if (smem_max > 227 * 1024) smem_max = 227 * 1024;   // (plan_blocks keeps the tile within the per-block limit)
-  if (which == 3) {  // one-time: allow the dynamic shared memory the kernels need
+  if (which == 3) {  // one-time, on the handle's device: allow the dynamic shared memory the kernels need
     cudaError_t e = cudaFuncSetAttribute(k_step<AC, BC, HC, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_reset<AC, BC, HC, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_observe<AC, BC, HC, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
+    if (e == cudaSuccess) e = obs_attrs<false>();
+    if (e == cudaSuccess) e = obs_attrs<true>();
     return e;
   }
   if (which == 0 && C.pdl_wait) {
@@ -768,34 +700,21 @@ cudaError_t msv_launch_truncate(const DevConst& C, const DevState& S, const DevO
 }
 
 cudaError_t msv_launch_obs(const DevConst& C, const DevState& S, const ObsTable& T, int AC, const uint8_t* only_if, cudaStream_t st) {
-#ifndef MSV_OBS_GENERIC
-  if (!only_if) {                                // every row: the source-major kernel
-    size_t smem = 0;
-    for (int k = 0; k < MSV_OBS_KEYS; ++k) smem += (size_t)OBS2_E * T.keys[k].chunk * sizeof(float);
-    static bool attr_set = false;
-    if (!attr_set) {
-      cudaFuncSetAttribute(k_obs2, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-      // same L1/shared split as the step kernel, so that a tile can become resident on an SM that still runs one of its blocks
-      const char* cv = getenv("MSV_OBS_CARVEOUT");
-      if (!cv || atoi(cv) != 0) cudaFuncSetAttribute(k_obs2, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-      attr_set = true;
-    }
-    // one warp per source item when they fit a block (a single round of loads), else 32 warps looping over the items
-    const int n_items = C.A + 2 * C.B0 + C.H0 + 1;
-    const int threads = n_items <= 32 ? 32 * n_items : 1024;
-    const int spb = (C.epb + OBS2_E - 1) / OBS2_E;                       // tiles per k_step block
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)((C.N / C.epb) * spb)); cfg.blockDim = dim3((unsigned)threads);
-    cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;                // may start before the step kernel has finished
-    cfg.attrs = at; cfg.numAttrs = C.tq_ticket ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, k_obs2, C, S, T, AC);
-  }
-#endif
-  k_obs<<<(C.n_real + OBS_EPB - 1) / OBS_EPB, 256, (size_t)OBS_EPB * T.n_elems * sizeof(float), st>>>(C, S, T, AC, only_if);
-  return cudaPeekAtLastError();
+  size_t smem = 0;
+  for (int k = 0; k < MSV_OBS_KEYS; ++k) smem += (size_t)OBS2_E * T.keys[k].chunk * sizeof(float);
+  // one warp per source item when they fit a block (a single round of loads), else 32 warps looping over the items
+  const int n_items = C.A + 2 * C.B0 + C.H0 + 1;
+  const int threads = n_items <= 32 ? 32 * n_items : 1024;
+  const int spb = (C.epb + OBS2_E - 1) / OBS2_E;                       // tiles per k_step block
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)((C.N / C.epb) * spb)); cfg.blockDim = dim3((unsigned)threads);
+  cfg.dynamicSmemBytes = smem; cfg.stream = st;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;                // may start before the step kernel has finished
+  cfg.attrs = at; cfg.numAttrs = C.tq_ticket ? 1 : 0;
+  if (only_if) return cudaLaunchKernelEx(&cfg, k_obs2<true>, C, S, T, AC, only_if);
+  return cudaLaunchKernelEx(&cfg, k_obs2<false>, C, S, T, AC, only_if);
 }
 
 cudaError_t msv_launch_lidar(const DevConst& C, const DevState& S, const DevOut& O, int BC, int HC, cudaStream_t st) {

@@ -24,6 +24,7 @@ cudaError_t msv_read_blocks(unsigned long long* out, int n_words);
 cudaError_t msv_read_trace(unsigned long long* out, int n_words);
 cudaError_t msv_read_check(unsigned long long out[2]);
 cudaError_t msv_launch_spare(const DevConst& C, const DevState& S, const uint8_t* dones, int only_done, cudaStream_t st);
+// k_obs2 into T's tensors: every row (only_if NULL), or the rows of the real envs whose only_if byte is set
 cudaError_t msv_launch_obs(const DevConst& C, const DevState& S, const ObsTable& T, int AC, const uint8_t* only_if, cudaStream_t st);
 cudaError_t msv_launch_lidar(const DevConst& C, const DevState& S, const DevOut& O, int BC, int HC, cudaStream_t st);
 // msv_render: picture of envs [first, first+count) into out (uint8[count][H][W][3]); BC, HC the list capacities,

@@ -122,19 +122,10 @@ struct DevOut {
   uint8_t* br_results;   // [N][A]  BattleRoyale.results (valid where br_over)
 };
 
-// ---- observation writer (k_obs) ------------------------------------------
-// One thread per output float.  The host flattens every observation key of
-// the config into a table of element descriptors (what to read, from which
-// slot/component, under which validity condition) so the kernel is a pure
-// gather from the SoA state with fully coalesced stores.
-enum ObsSrc : uint8_t {
-  OS_ZERO = 0, OS_AGENT_ID, OS_AGENT_TEAM, OS_AGENT_HEALTH, OS_AKIN0, OS_AKIN1, OS_OTHERS_MASK,
-  OS_ZONE_CUR, OS_ZONE_NEXT, OS_HEAL, OS_LIST_MASK, OS_HEAL_SLOT, OS_HEAL_SLOT_MASK,
-  OS_BOX_VERT, OS_BOX_POS, OS_ITEM_VERT, OS_ITEM_POS, OS_BOX_SLOT, OS_BOX_SLOT_MASK
-};
-struct ObsDesc { uint8_t src, slot, comp, aux; uint16_t key; uint16_t off; };
+// ---- observation writer (k_obs2) -----------------------------------------
+// The observation keys in DevOut order (agent .. box_slot_mask): tensor base and floats per environment.
 struct ObsKey { float* base; int chunk; };
 #define MSV_OBS_KEYS 14
-// desc: elements in output order (key, offset).  cdesc: the same elements sorted by source kind,
-// `key` holding the element's index in `desc` -- warps of the compute phase are homogeneous.
-struct ObsTable { const ObsDesc* desc; const ObsDesc* cdesc; int n_elems; ObsKey keys[MSV_OBS_KEYS]; };
+struct ObsTable { ObsKey keys[MSV_OBS_KEYS]; };
+// keys 4-7 (heals ..) exist only with heals, keys 8-13 (boxes ..) only with boxes
+__host__ __device__ inline bool obs_key_used(int k, int H, int B) { return !((k >= 4 && k <= 7 && H == 0) || (k >= 8 && B == 0)); }

@@ -218,7 +218,7 @@ class Handle:
 
     def kernel_timing(self, enable):
         """debug: start (True) / stop (False) CUDA-event timing of the kernels of step(); stopping
-        returns (mean ms of [k_step, k_obs, k_lidar], number of steps recorded)."""
+        returns (mean ms of [k_step, k_obs2, k_lidar], number of steps recorded)."""
         out = (ctypes.c_double * 3)()
         n = ctypes.c_int64()
         check(load().msv_debug_kernel_timing(self.h, 1 if enable else 0, out, ctypes.byref(n)), self.h)

@@ -353,7 +353,7 @@ int msv_flush_stats(msv_handle* h, msv_stats* out);
  * its split by kernel (which: 0 step kernel, 1 observation gather, 2 lidar). */
 int64_t msv_bytes_per_env_step(msv_handle* h);
 int64_t msv_kernel_bytes_per_env(msv_handle* h, int32_t which);
-/* The part of it written by the observation gather kernel (k_obs). */
+/* The part of it written by the observation kernel (k_obs2). */
 int64_t msv_obs_bytes_per_env(msv_handle* h);
 int64_t msv_kernel_launches(msv_handle* h); /* launches since create */
 /* How the batch is tiled onto the GPU: out[0] environments per thread block of

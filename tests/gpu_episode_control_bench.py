@@ -1,8 +1,10 @@
-"""Cost of the step limit and of msv_reset_envs on the 2v2 workload (16 384 environments, auto_reset=True).
-  (a) ms per step with max_episode_steps T = 0, 300 and 10**6.  The three handles are pre-rolled to the stationary
-      episode mix (--preroll steps each, as bench.py does) and timed in alternating blocks of --steps steps
-      (CUDA events around each block); the median block over --rounds rounds is reported.  T = 0 runs the tile
-      hand-off; T > 0 gives it up and adds k_truncate and the k_reset of the finished environments.
+"""Cost of the step limit, of terminal capture and of msv_reset_envs on the 2v2 workload (16 384 environments).
+  (a) ms per step with auto_reset=True and max_episode_steps T = 0, 300 and 10**6, and with auto_reset='terminal'
+      and T = 0 and 300.  The five handles are pre-rolled to the stationary episode mix (--preroll steps each, as
+      bench.py does) and timed in alternating blocks of --steps steps (CUDA events around each block); the median
+      block over --rounds rounds is reported.  auto_reset=True with T = 0 runs the tile hand-off; the other cases
+      give it up and add k_truncate (T > 0), the row-filtered k_obs2 into terminal_* (terminal) and the k_reset
+      of the finished environments.
   (b) device-event time of one reset_envs with 1 %, 10 % and 100 % of the environments masked (mean over --iters
       calls, one untimed step between calls).
 Each handle's state and outputs (about 100 MB) largely fit the 126 MB L2, unlike bench.py's rotating batches.
@@ -46,43 +48,43 @@ def main():
     acts = [torch.randint(0, 2, (N, 4, 6), dtype=torch.uint8, device='cuda:0', generator=g) for _ in range(16)]
     for a in acts:
         a[..., :3] = torch.randint(0, 3, (N, 4, 3), dtype=torch.uint8, device='cuda:0', generator=g)
-    limits = (0, 300, 10 ** 6)
-    envs = {T: MaSurvivalVec(variant('2v2'), N, seed=1, auto_reset=True, max_episode_steps=T) for T in limits}
-    k = {T: 0 for T in limits}
+    cases = ((True, 0), (True, 300), (True, 10 ** 6), ('terminal', 0), ('terminal', 300))    # (auto_reset, T)
+    envs = {c: MaSurvivalVec(variant('2v2'), N, seed=1, auto_reset=c[0], max_episode_steps=c[1]) for c in cases}
+    k = {c: 0 for c in cases}
 
-    def step(T):
-        envs[T].step(acts[k[T] % len(acts)])
-        k[T] += 1
-    for T in limits:
-        envs[T].reset()
+    def step(c):
+        envs[c].step(acts[k[c] % len(acts)])
+        k[c] += 1
+    for c in cases:
+        envs[c].reset()
         for _ in range(args.preroll):
-            step(T)
+            step(c)
     torch.cuda.synchronize()
-    blocks = {T: [] for T in limits}
+    blocks = {c: [] for c in cases}
     t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     for _ in range(args.rounds):
-        for T in limits:
+        for c in cases:
             t0.record()
             for _ in range(args.steps):
-                step(T)
+                step(c)
             t1.record()
             torch.cuda.synchronize()
-            blocks[T].append(t0.elapsed_time(t1) / args.steps)
+            blocks[c].append(t0.elapsed_time(t1) / args.steps)
     rows = []
-    for T in limits:
-        b = sorted(blocks[T])
-        row = {'case': 'step', 'workload': '2v2', 'envs': N, 'max_episode_steps': T, 'ms_per_step': round(b[len(b) // 2], 5),
-               'min': round(b[0], 5), 'max': round(b[-1], 5), 'blocks': len(b), 'steps_per_block': args.steps,
-               'hand_off': envs[T].tile_plan()['observation_hand_off'], 'card': gpu}
+    for c in cases:
+        b = sorted(blocks[c])
+        row = {'case': 'step', 'workload': '2v2', 'envs': N, 'auto_reset': c[0], 'max_episode_steps': c[1],
+               'ms_per_step': round(b[len(b) // 2], 5), 'min': round(b[0], 5), 'max': round(b[-1], 5), 'blocks': len(b),
+               'steps_per_block': args.steps, 'hand_off': envs[c].tile_plan()['observation_hand_off'], 'card': gpu}
         print(json.dumps(row), flush=True)
         rows.append(row)
-    env = envs[0]
+    env = envs[(True, 0)]
     rng = np.random.default_rng(2)
     for frac in (0.01, 0.10, 1.0):
         mask = torch.as_tensor(rng.random(N) < frac if frac < 1 else np.ones(N, bool)).cuda()
         tot = 0.0
         for i in range(args.iters + 5):
-            step(0)
+            step((True, 0))
             t0.record()
             env.reset_envs(mask)
             t1.record()

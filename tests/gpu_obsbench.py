@@ -1,4 +1,4 @@
-"""Times k_obs alone (observe_only) and the step kernel alone for the 2v2 workload."""
+"""Times k_obs2 alone (observe_only) and the step kernel alone for the 2v2 workload."""
 import torch
 import parity
 from parity import make_config
@@ -15,7 +15,7 @@ e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=Tr
 e0.record()
 for t in range(200): h.observe_only()
 e1.record(); torch.cuda.synchronize()
-print('k_obs %.1f us' % (e0.elapsed_time(e1) / 200 * 1e3))
+print('k_obs2 %.1f us' % (e0.elapsed_time(e1) / 200 * 1e3))
 e0.record()
 for t in range(200): h.step_kernel_only(acts[t % 8].data_ptr())
 e1.record(); torch.cuda.synchronize()

@@ -50,6 +50,25 @@ MATRIX = [
 ]
 LANES = {0: 2, 1: 4, 2: 8}
 
+# the observation tensors the library stores (msv_tensor_info names), lidar aside
+OBS_KEYS = ('agent', 'others', 'others_mask', 'zone', 'heals', 'heals_mask', 'heal_slot', 'heal_slot_mask',
+            'boxes', 'boxes_mask', 'box_items', 'box_items_mask', 'box_slot', 'box_slot_mask')
+
+
+def terminal_snapshot(h):
+    """copies of a terminal-mode handle's terminal_<key> observation tensors (terminal_lidar_* left out:
+    the terminal k_lidar rewrites every row on every step)"""
+    names = ['terminal_' + k for k in OBS_KEYS]
+    return {n: h.tensor(n).clone() for n in names if h.has_tensor(n)}
+
+
+def assert_unfinished_rows_kept(h, snap, finished, where=None):
+    """the rows of environments that did not finish on the step are the bytes they held before it"""
+    import torch
+    keep = torch.as_tensor(finished).to('cuda') == 0
+    for n, before in snap.items():
+        assert torch.equal(h.tensor(n)[keep].view(torch.int32), before[keep].view(torch.int32)), (where, n)
+
 
 def matrix_config(over, auto_reset=False, fast=True):
     return make_config('1v1', auto_reset=auto_reset, **_merge(FAST if fast else {}, over))

@@ -202,7 +202,9 @@ def test_terminal_capture_matrix(name, over, cls, N):
     for t in range(100):
         act = random_actions(rng, N, A)
         a = torch.as_tensor(act).cuda()
+        snap = oc.terminal_snapshot(et._h)
         ot, rt, dt, info = et.step(a)
+        oc.assert_unfinished_rows_kept(et._h, snap, dt, t)
         o1, r1, d1, _ = e1.step(a)
         for k in o1:
             assert torch.equal(ot[k], o1[k]), (t, k)

@@ -289,7 +289,10 @@ def test_step_limit_lockstep(name, N, T, mode):
     rng = np.random.default_rng(seed)
     for t in range(80):
         act = random_actions(rng, N, A)
+        before = oc.terminal_snapshot(env._h) if mode == 'terminal' else None
         _, _, d, info = env.step(torch.as_tensor(act).cuda())
+        if before is not None:
+            oc.assert_unfinished_rows_kept(env._h, before, d | info['truncated'], t)
         g, sg = _snapshot(env._h, names), env.get_state()
         tr = info['truncated'].cpu().numpy()
         term = {k: v.cpu().numpy() for k, v in info['terminal_observation'].items()} if mode == 'terminal' else None

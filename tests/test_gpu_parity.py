@@ -3,13 +3,20 @@ oracle on identical seeded inputs.  Discrete outputs (health, inventories,
 alive/done flags, masks, rewards, lidar hit ids, contact bookkeeping) must be
 bit-exact; continuous outputs within 1e-4 relative (BASELINE.json north_star).
 In practice every field is bit-exact and the tests also assert that."""
+import math
+
 import numpy as np
 import pytest
 
+import obs_cases as oc
 import parity
 from parity import compare_obs, compare_states, make_config, random_actions, scramble_state
 
 pytestmark = pytest.mark.gpu
+
+# every output tensor of a step besides the terminal-mode copies
+OUTPUTS = oc.OBS_KEYS + ('lidar_frac', 'lidar_hit', 'rewards', 'dones', 'episode_return', 'episode_length', 'immune',
+                         'br_over', 'br_results', 'truncated')
 
 
 def _assert_clean(r, need_exact=True):
@@ -338,6 +345,7 @@ def test_abi_tensor_info_errors_and_lifetime():
     assert t.shape == (100, 8, 8) and t.is_cuda and t.data_ptr() == h.tensor('agent').data_ptr()
     assert h.tensor('lidar_hit').dtype == torch.int32 and h.tensor('dones').dtype == torch.uint8
     assert h.bytes_per_env_step() > h.obs_bytes_per_env() > 0
+    assert h.obs_bytes_per_env() == 4 * _stored_obs_floats(h)
     # checkpoint / resume: get_state -> set_state is the identity, and a restored env continues identically
     a = torch.zeros((100, 8, 6), dtype=torch.uint8, device='cuda'); a[..., :3] = 2; a[..., 3] = 1
     for _ in range(25):
@@ -357,6 +365,55 @@ def test_abi_tensor_info_errors_and_lifetime():
     with pytest.raises(_lib.MasurvError):
         h.get_state(first=100, count=1)
     h.close()
+    # the observation bytes per env are the stored observation tensors, for every agent count, class, H = 0 and B = 0
+    recs = [oc.matrix_config(m[2]) for m in oc.MATRIX] + [make_config(n) for n in ('2v2', 'ffa', '1v1_heal_only')]
+    recs.append(make_config('1v1', **{k: dict(v) for k, v in parity.EXOTIC_B.items()}))
+    for rec in recs:
+        h = _lib.Handle(rec, 37, 0, 1, 0)
+        assert h.obs_bytes_per_env() == 4 * _stored_obs_floats(h), rec
+        h.close()
+
+
+def _stored_obs_floats(h):
+    """floats per environment of the observation tensors as msv_tensor_info shapes them (zone, heals, boxes and
+    box_items are stored once per env; a key the config does not have counts 0)"""
+    import ctypes
+    from masurvival import _lib
+    nd, shape, n = ctypes.c_int32(), (ctypes.c_int64 * 4)(), 0
+    for k in oc.OBS_KEYS:
+        if _lib.load().msv_tensor_info(h.h, k.encode(), None, ctypes.byref(nd), shape, None, None) == 0:
+            n += math.prod(shape[1:nd.value])
+    return n
+
+
+def test_two_devices_in_one_process():
+    """The same ffa batch (8-lane class: the largest observation stage) on device 0 and device 1 of one process,
+    stepped with the same actions, gives the same outputs: each handle prepares its kernels on its own device."""
+    import torch
+    from masurvival import _lib
+    if torch.cuda.device_count() < 2:
+        pytest.skip('needs two visible devices')
+    rec = make_config('ffa', auto_reset=True)
+    N, A = 100, int(rec['n_agents'])
+    hs = [_lib.Handle(rec, N, d, 3, 0) for d in (0, 1)]
+    assert [h.tile_plan()['threads_per_block'] // h.tile_plan()['envs_per_block'] for h in hs] == [8, 8]
+    names = [n for n in OUTPUTS if hs[0].has_tensor(n)]
+    for d, h in enumerate(hs):
+        with torch.cuda.device(d):
+            h.reset()
+    rng = np.random.default_rng(3)
+    for t in range(40):
+        act = random_actions(rng, N, A)
+        for d, h in enumerate(hs):
+            a = torch.as_tensor(act).to(f'cuda:{d}')
+            with torch.cuda.device(d):
+                h.step(a.data_ptr())
+            torch.cuda.synchronize(d)
+        for n in names:
+            assert torch.equal(hs[0].tensor(n).cpu(), hs[1].tensor(n).cpu()), (t, n)
+    assert hs[0].get_state().tobytes() == hs[1].get_state().tobytes()
+    for h in hs:
+        h.close()
 
 
 def test_step_host_obs_and_async_pipeline():
