@@ -56,7 +56,7 @@ struct msv_handle {
   // back into the caller's stream before msv_step returns (fork/join inside the call: graph-capture safe)
   cudaStream_t side_stream = nullptr; cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   uint32_t tq_ticket = 0, tq_base = 0; bool handoff = true;   // k_step -> k_obs2 tile hand-off (MSV_NO_HANDOFF=1 turns it off)
-  bool step_pdl = true, last_was_step = false, no_spare = false; cudaStream_t last_stream = nullptr;   // k_step programmatically dependent on the previous step's observation kernel (MSV_STEP_PDL=0 turns it off)
+  bool last_was_step = false; cudaStream_t last_stream = nullptr;   // the last call on last_stream ended with the hand-off's observation kernel: the next k_step is programmatically dependent on it
   // debug: CUDA-event timing of the kernels of msv_step (bench.py's roofline numerator)
   bool timing = false; std::vector<cudaEvent_t> tev; size_t tev_used = 0;
   double* d_stat_reward; unsigned long long* d_stat_kills; unsigned long long* d_stat_misc;
@@ -419,8 +419,6 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
   msv_capacity(h->cap, &h->AC, &h->BC, &h->HC, &h->P, &h->PW, &h->sm_words);
   plan_blocks(h, device);
   if (const char* nh = getenv("MSV_NO_HANDOFF")) h->handoff = atoi(nh) == 0;   // development A/B: plain stream-ordered launches
-  if (const char* sp = getenv("MSV_STEP_PDL")) h->step_pdl = atoi(sp) != 0;
-  if (const char* ns = getenv("MSV_NO_SPARE")) h->no_spare = atoi(ns) != 0;    // development: no record kernel (resets draw their own)
   if (msv_launch(h->cap, 3, h->C, h->S, h->O, nullptr, 0) != cudaSuccess) {
     g_err = "cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed"; delete h; return MSV_ERR_CUDA;
   }
@@ -649,7 +647,7 @@ static int launch(msv_handle* h, int which, const uint8_t* dev_in, void* stream)
   if (handoff) {
     if (++h->tq_ticket == 0u) h->tq_ticket = 1u;
     Cq.tq_ticket = h->tq_ticket; Cq.tq_base = h->tq_base;
-    Cq.pdl_wait = (h->step_pdl && h->last_was_step && h->last_stream == st) ? 1u : 0u;   // the previous call on this stream ended with this handle's observation kernels
+    Cq.pdl_wait = (h->last_was_step && h->last_stream == st) ? 1u : 0u;   // the previous call on this stream ended with this handle's observation kernels
     h->tq_base += (uint32_t)(h->C.N / h->C.epb);
   }
   if (split) {
@@ -691,7 +689,7 @@ static int launch(msv_handle* h, int which, const uint8_t* dev_in, void* stream)
   if (timed) tmark(h, st);
   if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O, h->BC, h->HC, (cudaStream_t)stream)); h->launches++; }
   if (timed) tmark(h, st);
-  const bool spare = (which == 1 || (which == 0 && h->cfg.auto_reset != 0)) && !h->no_spare;
+  const bool spare = which == 1 || (which == 0 && h->cfg.auto_reset != 0);
   if (spare) {                                  // the step / reset left finished environments without a record for their next episode
     if (!h->side_stream) {
       CK(cudaStreamCreateWithFlags(&h->side_stream, cudaStreamNonBlocking));

@@ -385,7 +385,7 @@ __device__ unsigned long long g_dbg[8];
 // 1 TOI event, 2 reset, 3 deaths, 4 pickups, 5 use/give, 6 contact numbering, 7 box removal)
 __device__ unsigned long long g_cnt[16];
 __device__ unsigned long long g_sub[16];   // sub-phase cycle sums inside toi_event (development)
-__device__ unsigned long long g_toi[16];   // the longest solve_toi call since the last read: [0] cycles, [1] loop iterations, [2] events run, [3] not touching, [4] identical repeats, [5] cycles in events, [6] cycles in scans, [7] b2TimeOfImpact calls dealt out
+__device__ unsigned long long g_toi[16];   // the longest solve_toi call since the last read: [0] cycles, [1] loop iterations, [2] events run, [3] not touching, [4] identical repeats, [5] cycles in events, [6] cycles in scans
 #define TOIPROF(x) x
 #define SUB_BEGIN() long long sub_t_ = clock64()
 #define SUB(k) do { long long n_ = clock64(); atomicAdd(&g_sub[k], (unsigned long long)(n_ - sub_t_)); sub_t_ = n_; } while (0)

@@ -74,42 +74,6 @@ struct BodyS { f2 c; float a; f2 v; float w; float invM, invI; };
 // the block's dynamic shared memory (addressed as shared, not through a generic pointer)
 extern __shared__ float msv_sm[];
 
-
-#ifndef MSV_INLINE_MASK
-#define MSV_INLINE_MASK 0
-#endif
-#ifndef MSV_TOI_COOP
-#define MSV_TOI_COOP 0   // deal the b2TimeOfImpact calls of SolveTOI out to the group's lanes (0: every lane its own agent's)
-#endif
-#ifndef MSV_FIXPOINT
-#define MSV_FIXPOINT 1   // stop Gauss-Seidel sweeps at a bitwise fixed point (exact); 0 = always run every iteration (development A/B)
-#endif
-#if (MSV_INLINE_MASK >> 0) & 1
-#define COLD0 __device__ __forceinline__
-#else
-#define COLD0 __device__ __noinline__
-#endif
-#if (MSV_INLINE_MASK >> 1) & 1
-#define COLD1 __device__ __forceinline__
-#else
-#define COLD1 __device__ __noinline__
-#endif
-#if (MSV_INLINE_MASK >> 2) & 1
-#define COLD2 __device__ __forceinline__
-#else
-#define COLD2 __device__ __noinline__
-#endif
-#if (MSV_INLINE_MASK >> 3) & 1
-#define COLD3 __device__ __forceinline__
-#else
-#define COLD3 __device__ __noinline__
-#endif
-#if (MSV_INLINE_MASK >> 4) & 1
-#define COLD4 __device__ __forceinline__
-#else
-#define COLD4 __device__ __noinline__
-#endif
-
 // Counter-based Philox draws of (global env id, episode, step, stream, block): two uniform doubles per block
 __device__ __noinline__ double2 philox_uniform2_of(const DevConst& C, uint32_t genv, uint32_t episode, uint32_t step, uint32_t stream, uint32_t blk) {
   uint32_t o[4];
@@ -253,12 +217,6 @@ struct Env {
     for (int w = 0; w < PW; ++w) { ex[w] = o.ex[w]; tc[w] = o.tc[w]; en[w] = o.en[w]; }
   }
 #define MSV_COLD(call) do { Env c_(*this); c_.call; take(c_); } while (0)
-  // MSV_INLINE_MASK (development): bit k set -> the cold functions of class k are inlined into the
-  // kernel instead (0 islands, 1 TOI events, 2 contact numbering, 3 deaths/pickups/use-give/box removal, 4 reset)
-#ifndef MSV_INLINE_MASK
-#define MSV_INLINE_MASK 0
-#endif
-#define MSV_COLDK(k, call) do { if ((MSV_INLINE_MASK >> (k)) & 1) { call; } else { Env c_(*this); c_.call; take(c_); } } while (0)
 
   // ---- shared-memory accessors
   DEV float& AG(int f, int i) { return msv_sm[sb + (CHK_IDX(f, F_COUNT) * AC + CHK_IDX(i, AC))]; }
@@ -521,7 +479,7 @@ struct Env {
 
   // ---- list maintenance (stable compaction, sim:185-189)            [leader]
   // shift the AB pair column k+1.. down by one for every agent
-  COLD3 void remove_box(int k) {
+  __device__ __noinline__ void remove_box(int k) {
     for (int i = 0; i < C.A; ++i) {   // b2World::DestroyBody -> contacts die, touching ones wake
       int p = p_ab(i, k);
       if (bit(ex, p) && bit(tc, p)) wake(i);
@@ -612,7 +570,7 @@ struct Env {
     }
   }
   // [leader] create the candidate contacts in proxy-pair order
-  COLD2 void number_candidates(unsigned long long* cand) {
+  __device__ __noinline__ void number_candidates(unsigned long long* cand) {
     for (;;) {
       int best = -1; unsigned bestKey = 0xFFFFFFFFu;
       for (int w = 0; w < PW; ++w) {
@@ -654,7 +612,7 @@ struct Env {
           setb(ex, p); setb(en, p); clrb(tc, p);
           S.pseq[p * N + e] = (uint32_t)(++LI(L_CONTACTSEQ));
           S.pimp[p * N + e] = make_float2(0.0f, 0.0f);
-        } else { RARE_BEGIN(); unsigned long long cc[PW]; for (int w = 0; w < PW; ++w) cc[w] = cand[w]; MSV_COLDK(2, number_candidates(cc)); RARE_END(6); }
+        } else { RARE_BEGIN(); unsigned long long cc[PW]; for (int w = 0; w < PW; ++w) cc[w] = cand[w]; MSV_COLD(number_candidates(cc)); RARE_END(6); }
       }
       share_bits();
     }
@@ -1000,7 +958,7 @@ struct Env {
           solve_velocity_static(nrm[k], rB[k], nm[k], tm[k], ni_[k], ti_[k], vB, wB);
           changed |= (__float_as_uint(ni_[k]) != __float_as_uint(n0)) | (__float_as_uint(ti_[k]) != __float_as_uint(t0));
         }
-        if (MSV_FIXPOINT && !changed && __float_as_uint(vB.x) == __float_as_uint(v_in.x) && __float_as_uint(vB.y) == __float_as_uint(v_in.y) &&
+        if (!changed && __float_as_uint(vB.x) == __float_as_uint(v_in.x) && __float_as_uint(vB.y) == __float_as_uint(v_in.y) &&
             __float_as_uint(wB) == __float_as_uint(w_in)) break;
       }
 #pragma unroll (NRr <= NR ? NRr : 1)
@@ -1151,7 +1109,7 @@ struct Env {
         }
         changed |= (__float_as_uint(ni_[k]) != __float_as_uint(n0_)) | (__float_as_uint(ti_[k]) != __float_as_uint(t0_));
       }
-      if (MSV_FIXPOINT && it >= 0 && !changed &&
+      if (it >= 0 && !changed &&
           __float_as_uint(vX.x) == __float_as_uint(vX_in.x) && __float_as_uint(vX.y) == __float_as_uint(vX_in.y) && __float_as_uint(wX) == __float_as_uint(wX_in) &&
           __float_as_uint(vY.x) == __float_as_uint(vY_in.x) && __float_as_uint(vY.y) == __float_as_uint(vY_in.y) && __float_as_uint(wY) == __float_as_uint(wY_in)) break;
     }
@@ -1203,7 +1161,7 @@ struct Env {
     }
     synchronize_fixtures(X); synchronize_fixtures(Y);
   }
-  COLD0 void solve_island(int seed, float h, float dtRatio) {
+  __device__ __noinline__ void solve_island(int seed, float h, float dtRatio) {
     SUB_BEGIN();
     Ord ord; ord.lo = 0ull; ord.hi = 0ull;
     int nc = 0; unsigned taken = 0, inisl = 1u << seed;
@@ -1431,7 +1389,7 @@ struct Env {
       }
       if (comp == (1u << i)) { solve_single(i, h, dtRatio); continue; }
       const unsigned cand = comp & awk;          // no awake member: the island is not simulated
-      if (cand != 0u && (31 - __clz((int)cand)) == i) { RARE_BEGIN(); SUB_BEGIN(); MSV_COLDK(0, solve_island(i, h, dtRatio)); SUBMAX(13, __popc(comp)); RARE_END(0); }
+      if (cand != 0u && (31 - __clz((int)cand)) == i) { RARE_BEGIN(); SUB_BEGIN(); MSV_COLD(solve_island(i, h, dtRatio)); SUBMAX(13, __popc(comp)); RARE_END(0); }
     }
     gsync();
   }
@@ -1464,7 +1422,7 @@ struct Env {
   static constexpr int TOI_ISL = 8;
   static_assert(SNAPW <= K_COUNT * (MAXC - TOI_ISL), "snapshot does not fit the scratch slots");
   DEV unsigned& SNAP(int q) { CHK((unsigned)q < (unsigned)SNAPW); return reinterpret_cast<unsigned*>(msv_sm)[sb + (W_TC + (q / (MAXC - TOI_ISL)) * MAXC + TOI_ISL + q % (MAXC - TOI_ISL))]; }
-  COLD1 int toi_event(int minP, float minAlpha, float dt, int prevP) {
+  __device__ __noinline__ int toi_event(int minP, float minAlpha, float dt, int prevP) {
     SUB_BEGIN();
     int a, sid, b; decode(minP, a, sid, b);
     // backup the agent's sweep, advance to the TOI, re-evaluate the contact
@@ -1616,13 +1574,11 @@ struct Env {
       const float alpha0 = AG(F_ALPHA0, j);
       return state == TOI_TOUCHING ? fmin_(alpha0 + (1.0f - alpha0) * beta, 1.0f) : 1.0f;
     };
-    TOIPROF(long long tp0 = clock64(); long long tp_ev = 0; int tp_it = 0; int tp_ran = 0; int tp_not = 0; int tp_same = 0; int tp_calls = 0;)
+    TOIPROF(long long tp0 = clock64(); long long tp_ev = 0; int tp_it = 0; int tp_ran = 0; int tp_not = 0; int tp_same = 0;)
     for (int guard = 0; guard < 64; ++guard) {
       TOIPROF(tp_it++;)
       // ---- (1) every lane: the existing, enabled agent-vs-static contacts of its agent that still take part.
-      // Cached TOIs enter the minimum directly; the contacts whose TOI must be computed are collected in `need`
-      // (bit k = static body k).
-      unsigned need = 0u;
+      // Cached TOIs enter the minimum directly.
       int minP = -1, minSeq = -1; float minAlpha = 1.0f;
       // the world contact list is newest first and the scan keeps the FIRST minimum:
       // on equal alpha the contact with the larger creation sequence wins
@@ -1653,38 +1609,11 @@ struct Env {
             const float gx = fmax_(fmin_(l0.x, l1.x) - sbx.hx, -sbx.hx - fmax_(l0.x, l1.x));
             const float gy = fmax_(fmin_(l0.y, l1.y) - sbx.hy, -sbx.hy - fmax_(l0.y, l1.y));
             if (fmax_(gx, gy) > (B2_POLY_RADIUS + C.agent_r - 3.0f * B2_LINEAR_SLOP) + 0.25f * B2_LINEAR_SLOP + 0.004f) { TOIA(i, k) = 1.0f; cvalid |= 1u << k; }
-            else if (MSV_TOI_COOP) need |= 1u << k;
             else { const float al = toi_alpha(i, k); TOIA(i, k) = al; cvalid |= 1u << k; consider(p, al); }
           }
         }
       }
-      // ---- (2) the group computes the missing TOIs together: the calls are dealt out to the lanes in
-      // (agent, static body) order, so an agent wedged between several bodies does not serialise them on
-      // its own lane while the others idle.  Any lane can evaluate any pair: the inputs sit in shared memory.
-      if (MSV_TOI_COOP && __any_sync(gmask, need != 0u)) {          // group-uniform
-        unsigned ms[G]; int T = 0;
-#pragma unroll
-        for (int j = 0; j < G; ++j) { ms[j] = from(need, j); T += __popc(ms[j]); }
-        TOIPROF(tp_calls += T;)
-        for (int r0 = 0; r0 < T; r0 += G) {
-          const int t = r0 + g;
-          int fj = -1, fk = 0, base = 0;
-#pragma unroll
-          for (int j = 0; j < G; ++j) {
-            const int c = __popc(ms[j]);
-            if (t >= base && t < base + c) { fj = j; fk = (int)__fns(ms[j], 0u, t - base + 1); }
-            base += c;
-          }
-          if (fj >= 0) TOIA(fj, fk) = toi_alpha(fj, fk);
-        }
-        gsync();
-        cvalid |= need;
-        while (need) {
-          const int k = __ffs((int)need) - 1; need &= need - 1u;
-          consider(k < BC ? p_ab(i, k) : p_aw(i, k - BC), TOIA(i, k));
-        }
-      }
-      // ---- (3) minimum over the group
+      // ---- (2) minimum over the group
 #pragma unroll
       for (int o = 1; o < G; o <<= 1) {        // group minimum (alpha ascending, creation sequence descending)
         float oa = __shfl_xor_sync(gmask, minAlpha, o, G);
@@ -1700,8 +1629,7 @@ struct Env {
       TOIPROF(long long tpe = clock64();)
       if (lead) {
         RARE_BEGIN();
-        if ((MSV_INLINE_MASK >> 1) & 1) r = toi_event(minP, minAlpha, dt, prevP);
-        else { Env c_(*this); r = c_.toi_event(minP, minAlpha, dt, prevP); take(c_); }
+        Env c_(*this); r = c_.toi_event(minP, minAlpha, dt, prevP); take(c_);
         if (r & 1) prevP = minP;
         RARE_END(1);
       }
@@ -1726,7 +1654,7 @@ struct Env {
     }
     gsync();
     TOIPROF(if (lead) { unsigned long long tot = (unsigned long long)(clock64() - tp0); unsigned long long old = atomicMax(&g_toi[0], tot);
-      if (tot > old) { g_toi[1] = tp_it; g_toi[2] = tp_ran; g_toi[3] = tp_not; g_toi[4] = tp_same; g_toi[5] = (unsigned long long)tp_ev; g_toi[6] = tot - (unsigned long long)tp_ev; g_toi[7] = tp_calls; g_toi[8] = (unsigned long long)e; } })
+      if (tot > old) { g_toi[1] = tp_it; g_toi[2] = tp_ran; g_toi[3] = tp_not; g_toi[4] = tp_same; g_toi[5] = (unsigned long long)tp_ev; g_toi[6] = tot - (unsigned long long)tp_ev; g_toi[8] = (unsigned long long)e; } })
   }
 
   // ======================================================================
@@ -1760,9 +1688,9 @@ struct Env {
     bool any = LI(L_NP) > 0;                       // nothing to do unless a drop is pending or an agent with items uses/gives
 #pragma unroll
     for (int i = 0; i < AC; ++i) if (i < C.A && (((act >> (8 + i)) | (act >> (16 + i))) & 1u) && (LI(L_INV + (i)) & 7) != 0 && alive(i)) any = true;
-    if (any) { RARE_BEGIN(); MSV_COLDK(3, pre_use_give_body(act)); RARE_END(5); }
+    if (any) { RARE_BEGIN(); MSV_COLD(pre_use_give_body(act)); RARE_END(5); }
   }
-  COLD3 void pre_use_give_body(unsigned act) {
+  __device__ __noinline__ void pre_use_give_body(unsigned act) {
     // boxes/Object.pre_step (sem:853-856, 902-905): pending drops become items
     for (int q = 0; q < LI(L_NP); ++q) {
       float4 p0 = S.pend0[q * N + e];
@@ -1985,14 +1913,14 @@ struct Env {
           S.pend1[LI(L_NP) * N + e] = C.box_ownership ? b1.z : MSV_CAUSE_NONE;
           LI(L_NP)++;
         } else LI(L_OVERFLOW)++;
-        { RARE_BEGIN(); MSV_COLDK(3, remove_box(k)); RARE_END(7); }
+        { RARE_BEGIN(); MSV_COLD(remove_box(k)); RARE_END(7); }
         removed++;
       }
     }
   }
   // agents/Cameras.post_step (sim:333-334) runs between the two halves
   // [leader] agents/Health.post_step -> despawn(dead) (sem:429-448)
-  COLD3 void handle_deaths() {
+  __device__ __noinline__ void handle_deaths() {
     int total = 0;
     for (int i = 0; i < C.A; ++i) if ((LU(L_DMASK) >> i) & 1u) total += inv_n(i);
     int top = total;
@@ -2040,7 +1968,7 @@ struct Env {
     }
   }
   // [leader] agents/AutoPickup.post_step (sem:278-283) for agent i: bodies in creation order
-  COLD3 void pickup_agent(int i) {
+  __device__ __noinline__ void pickup_agent(int i) {
     const float r2 = C.pickup_r * C.pickup_r;
     f2 me = apos(i);
     int lastSeq = -1;
@@ -2085,7 +2013,7 @@ struct Env {
 #pragma unroll
         for (int i = 0; i < AC; ++i) if ((dm >> i) & 1u) carried += LI(L_INV + (i)) & 7;
         if (carried == 0) kill_agents_empty(dm);      // nothing to drop (the usual case): TrackKills + DestroyBody only
-        else { RARE_BEGIN(); MSV_COLDK(3, handle_deaths()); RARE_END(3); }
+        else { RARE_BEGIN(); MSV_COLD(handle_deaths()); RARE_END(3); }
         dflag = 1;
       }
     }
@@ -2104,7 +2032,7 @@ struct Env {
     }
     near = or32(near);
     if (!lead) return;
-    for (int i = 0; i < C.A; ++i) if ((near >> i) & 1u) { RARE_BEGIN(); MSV_COLDK(3, pickup_agent(i)); RARE_END(4); }
+    for (int i = 0; i < C.A; ++i) if ((near >> i) & 1u) { RARE_BEGIN(); MSV_COLD(pickup_agent(i)); RARE_END(4); }
     // agents/SafeZone.post_step (sem:758-768) + tick (sem:776-811)
     for (int i = 0; i < C.A; ++i) {
       if (!alive(i)) continue;
@@ -2258,7 +2186,7 @@ struct Env {
   // RandomizeBoxShapes (sem:97-120), ThickRoomWalls, SafeZone.post_reset
   // (sem:739-756).  The numpy Generator is replaced by counter-based
   // Philox4x32-10 keyed by (seed, global env id, episode).          [leader]
-  COLD4 void reset() {
+  __device__ __noinline__ void reset() {
     LI(L_EPISODE) += 1; LI(L_STEPS) = 0;
     // the episode's random draws: the record k_spare prepared, or (no record for this episode yet) drawn now.
     // It is staged in the dead touching-contact list of the environment's shared-memory column.

@@ -8,7 +8,6 @@
 // k_truncate: the step limit (truncated flags, finished mask) between k_step and the resets.
 // k_observe: fetch_observations only (after msv_set_state).
 // k_stats : flush_stats reduction.
-#include <cstdlib>
 #include "msv_env.cuh"
 #include "msv_launch.h"
 
@@ -40,24 +39,17 @@ __device__ unsigned long long g_blk[MSV_BLK_MAX * MSV_BLK_STAMPS];
 #define TRACE(row, idx) do { } while (0)
 #endif
 
-// thread -> (environment slot of the block, lane of the group)
+// a cold Env member function called on a copy of the environment (see MSV_COLD in msv_env.cuh)
+#define MSV_COLD_ON(env, call) do { auto c_ = env; c_.call; env.take(c_); } while (0)
 // keep the warps of a block in the same phase: they then share instruction-cache lines
-#define MSV_COLD_ON(env, call) do { if ((MSV_INLINE_MASK >> 4) & 1) { env.call; } else { auto c_ = env; c_.call; env.take(c_); } } while (0)
 // Which of the ten phase barriers are kept (bit k = PHASE_SYNC(k)), per capacity class.  Measured on the stationary
 // workloads with one 512-thread block per SM (profiles/r02_barriers.txt): without any barrier the step is 50 % slower
 // (163 against 109 us, 2v2); dropping single ones moves it by +-1 %; for the 2- and 4-lane classes dropping the two
 // between solve, FindNewContacts and SolveTOI (3 and 9: the lanes flow from the island solver into the TOI scan)
 // gains 2.5 % (108.7 -> 106.0 us), while the 8-lane class is fastest with all ten (345 against 349 us).
-#ifndef MSV_SYNC_MASK_ALL
 #define MSV_SYNC_MASK(G) ((G) >= 8 ? 0x3FF : 0x1F7)
-#else
-#define MSV_SYNC_MASK(G) (MSV_SYNC_MASK_ALL)     // development: make SYNCMASK=0x... (one mask for every class)
-#endif
-#ifdef MSV_NO_PHASE_SYNC
-#define PHASE_SYNC(k) do { } while (0)
-#else
 #define PHASE_SYNC(k) do { if ((MSV_SYNC_MASK(G) >> (k)) & 1) __syncthreads(); PROFW(k); BLK_STAMP(); } while (0)
-#endif
+// thread -> (environment slot of the block, lane of the group)
 #define MSV_GROUP_SETUP(G)                                                                       \
   const int es = threadIdx.x / (G), g = threadIdx.x % (G);                                       \
   const int e = blockIdx.x * (blockDim.x / (G)) + es;  /* C.N >= gridDim.x * environments per block */ \
@@ -631,8 +623,7 @@ static cudaError_t obs_attrs() {
   // the stage of the 8-agent class is ~1 000 floats x 32 environments, far over the 48 KB default
   cudaError_t e = cudaFuncSetAttribute(k_obs2<kRows>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
   // same L1/shared split as the step kernel, so that a tile can become resident on an SM that still runs one of its blocks
-  const char* cv = getenv("MSV_OBS_CARVEOUT");
-  if (e == cudaSuccess && (!cv || atoi(cv) != 0))
+  if (e == cudaSuccess)
     e = cudaFuncSetAttribute(k_obs2<kRows>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   return e;
 }

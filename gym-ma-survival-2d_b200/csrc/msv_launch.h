@@ -2,9 +2,7 @@
 // kernel launchers (msv_kernels.cu, msv_render.cu).
 #pragma once
 #include "msv_types.cuh"
-#ifndef MSV_TPB
 #define MSV_TPB 512   // maximum threads per block of k_step / k_reset / k_observe (the actual size is a runtime choice, see plan_blocks)
-#endif
 // cap: capacity class 0 = <2,4,4>, 1 = <4,4,4>, 2 = <8,8,16>; which: 0 step, 2 observe, 3 one-time kernel attribute setup
 cudaError_t msv_launch(int cap, int which, const DevConst& C, const DevState& S, const DevOut& O,
                        const uint8_t* actions, cudaStream_t st);

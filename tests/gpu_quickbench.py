@@ -48,7 +48,7 @@ def blocks(variant, N, warm=1500, launches=40):
         rc = L.msv_debug_blocks(h.h, buf.ctypes.data, buf.size)
         assert rc == 0, rc
         b = buf.reshape(2048, W).astype(np.int64)
-        toi_rows.append(b[2047, :9].copy()); b[2047] = 0
+        toi_rows.append(b[2047, [0, 1, 2, 3, 4, 5, 6, 8]]); b[2047] = 0   # g_toi word 7 is unused
         nb = int((b[:, 0] > 0).sum())
         b = b[:nb]
         n = int(b[0, 0])
@@ -66,7 +66,7 @@ def blocks(variant, N, warm=1500, launches=40):
     for i in range(len(ph_mean)):
         nm = BLK_PHASES[i] if i < len(BLK_PHASES) else str(i)
         print('   %-20s %10.0f %14.0f %16.0f' % (nm, ph_mean[i], ph_max[i], ph_maxany[i]))
-    print('   longest solve_toi call of each launch: cycles, loop iterations, events run, not touching, identical repeats, cycles in events, cycles in scans, TOI calls, env')
+    print('   longest solve_toi call of each launch: cycles, loop iterations, events run, not touching, identical repeats, cycles in events, cycles in scans, env')
     for r in toi_rows[:16]:
         print('     ', ' '.join(str(int(x)) for x in r))
     h.close()

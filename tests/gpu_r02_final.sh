@@ -12,7 +12,6 @@ for w in 2v2 ffa ffa_lidar 1v1_heal_only; do
   timeout 900 python bench.py --workload $w > $out/bench_${tag}_$w.json 2>> $out/${tag}.err; echo "bench $w rc=$?"
 done
 timeout 900 python bench.py --impl reference --steps 20 --warmup 5 > $out/bench_ref_${tag}_2v2.json 2>> $out/${tag}.err; echo "bench ref rc=$?"
-for lib in libmasurv.so libmasurv_m3FF.so; do MSV_LIB=$D/$lib QB_ROT=3 timeout 300 python tests/gpu_quickbench.py 1v1_heal_only 4096 300 1500 2>&1 | tail -1; done | tee $out/${tag}_1v1_mask.txt
 MSV_LIB=$D/libmasurv_prof.so timeout 300 python tests/gpu_quickbench.py --trace 2v2 16384 > $out/${tag}_trace_2v2.txt 2>&1
 MSV_LIB=$D/libmasurv_prof.so timeout 300 python tests/gpu_quickbench.py --blocks 2v2 16384 > $out/${tag}_blocks_2v2.txt 2>&1
 MSV_LIB=$D/libmasurv_prof.so timeout 300 python tests/gpu_quickbench.py --blocks ffa 8192 > $out/${tag}_blocks_ffa.txt 2>&1
