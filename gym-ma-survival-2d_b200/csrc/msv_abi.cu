@@ -27,7 +27,7 @@ typedef struct DLManagedTensor {
 } DLManagedTensor;
 }
 
-struct TensorInfo { void* ptr; int ndim; int64_t shape[4]; int dtype; /*0 f32, 1 u8, 2 i32*/ };
+struct TensorInfo { void* ptr; int ndim; int64_t shape[4]; int64_t strides[4]; int dtype; /*0 f32, 1 u8, 2 i32*/ };
 
 struct msv_handle {
   msv_config cfg;
@@ -65,6 +65,9 @@ struct msv_handle {
   int64_t obs_floats = 0;    // floats of one environment's observation keys (the keys the config has)
   ObsTable obs_term;         // auto_reset == 2: same table, writing the "terminal_<key>" tensors
   DevOut O_term;             // auto_reset == 2: O with the lidar pointers on the "terminal_lidar_*" tensors
+  // MSV_OBS_FLAT: k_obs2 writes "obs_flat" (and "terminal_obs_flat") through these; base NULL in the dict layout
+  ObsFlat flat = {nullptr, nullptr, 0}, flat_term = {nullptr, nullptr, 0};
+  int lidar_stride = 0;      // floats between two agents' rows of lidar_frac: L (dict) or D (flat)
   uint8_t* truncated = nullptr;   // max_episode_steps > 0: the "truncated" tensor [N]
   uint8_t* finished = nullptr;    // max_episode_steps > 0: dones | truncated of the last step [N] (k_truncate)
   int64_t exported;          // live DLPack exports
@@ -298,8 +301,17 @@ template <typename T> static int dalloc(msv_handle* h, T** p, size_t count) {
 static void reg(msv_handle* h, const char* name, void* ptr, int dtype, std::initializer_list<int64_t> shape) {
   TensorInfo t; t.ptr = ptr; t.ndim = (int)shape.size(); t.dtype = dtype;
   int i = 0; for (auto s : shape) t.shape[i++] = s;
+  int64_t st = 1;
+  for (i = t.ndim - 1; i >= 0; --i) { t.strides[i] = st; st *= t.shape[i]; }
   h->tensors[name] = t;
 }
+
+// the observation keys in k_obs2's order (ObsTable), and the order of their columns in a row of obs_flat
+static const char* const kObsNames[MSV_OBS_KEYS] = {"agent", "others", "others_mask", "zone", "heals", "heals_mask", "heal_slot",
+                                                    "heal_slot_mask", "boxes", "boxes_mask", "box_items", "box_items_mask", "box_slot", "box_slot_mask"};
+static const int kFlatOrder[MSV_OBS_KEYS] = {0, 3, 1, 2, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13};
+// zone, heals, boxes, box_items: the same for every observer, stored once per env in the dict layout
+static bool obs_key_shared(int k) { return k == 3 || k == 4 || k == 8 || k == 10; }
 
 // ---- AoS <-> SoA -----------------------------------------------------------
 struct Mirror {
@@ -397,7 +409,8 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
       cfg->n_agents + cfg->n_boxes + cfg->n_heals > cfg->grid_size * cfg->grid_size ||
       cfg->inv_slots < 1 || cfg->inv_slots > MSV_MAX_SLOTS || cfg->zone_n_radiuses + 1 > MSV_MAX_ZONES ||
       cfg->zone_phases > cfg->zone_n_radiuses + 1 || cfg->lidar_n < 0 || cfg->lidar_n > MSV_MAX_LASERS ||
-      cfg->zone_phases < 1 || cfg->max_episode_steps < 0 || env_offset < 0 || env_offset + (int64_t)num_envs > (int64_t)1 << 32)   // Philox counter word 0 is 32 bits
+      cfg->zone_phases < 1 || cfg->max_episode_steps < 0 || (cfg->obs_layout != MSV_OBS_DICT && cfg->obs_layout != MSV_OBS_FLAT) ||
+      cfg->reserved1 != 0 || env_offset < 0 || env_offset + (int64_t)num_envs > (int64_t)1 << 32)   // Philox counter word 0 is 32 bits
     return MSV_ERR_INVALID;
   {  // b2PolygonShape::Set welds vertices closer than its tolerance: a box that small is not a box any more (Box2D asserts);
      // the kernel treats every box analytically, so such configs are refused instead of simulated differently
@@ -437,32 +450,44 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
   rc |= dalloc(h, &S.pseq, P * N); rc |= dalloc(h, &S.pimp, P * N);
   rc |= dalloc(h, &S.sreward, AC * N); rc |= dalloc(h, &S.skills, AC * N); rc |= dalloc(h, &S.smisc, N);
   const size_t A = cfg->n_agents, B = cfg->n_boxes, H = cfg->n_heals, Sw = h->C.S, L = cfg->lidar_n;
+  const bool flat = cfg->obs_layout == MSV_OBS_FLAT;
+  // the flat row: agent, zone, others, others_mask, (heals, heals_mask, heal_slot, heal_slot_mask), (boxes, boxes_mask,
+  // box_items, box_items_mask, box_slot, box_slot_mask), lidar_frac
+  const size_t D = Sw + 6 + (A - 1) * Sw + (A - 1) + (H > 0 ? 3 * H + 2 : 0) + (B > 0 ? 23 * B + 9 : 0) + L;
+  h->lidar_stride = (int)(flat ? D : L);
   rc |= dalloc(h, &S.epret, AC * N);
   rc |= dalloc(h, &S.spare, N * (size_t)MSV_SPARE_W); rc |= dalloc(h, &S.spare_ep, N);
   {  // one arena for every output tensor, so that msv_step_host_obs reads the observations back in ONE copy
     struct Slot { void** p; size_t bytes; };
     const size_t f = sizeof(float);
-    Slot slots[] = {
+    std::vector<Slot> slots = {
       {(void**)&O.rewards, N * A * f}, {(void**)&O.dones, N}, {(void**)&O.episode_return, N * A * f},
       {(void**)&O.episode_length, N * sizeof(int)}, {(void**)&O.immune, N}, {(void**)&O.br_over, N}, {(void**)&O.br_results, N * A},
-      // ---- observation block (obs_begin .. obs_end)
-      {(void**)&O.agent, N * A * Sw * f}, {(void**)&O.others, N * A * (A - 1) * Sw * f}, {(void**)&O.others_mask, N * A * (A - 1) * f},
-      {(void**)&O.zone, N * 6 * f}, {(void**)&O.heals, N * H * 2 * f}, {(void**)&O.heals_mask, N * A * H * f},
-      {(void**)&O.heal_slot, N * A * f}, {(void**)&O.heal_slot_mask, N * A * f}, {(void**)&O.boxes, N * B * 11 * f},
-      {(void**)&O.boxes_mask, N * A * B * f}, {(void**)&O.box_items, N * B * 10 * f}, {(void**)&O.box_items_mask, N * A * B * f},
-      {(void**)&O.box_slot, N * A * 8 * f}, {(void**)&O.box_slot_mask, N * A * f},
-      {(void**)&O.lidar_frac, N * A * L * f}, {(void**)&O.lidar_hit, N * A * L * sizeof(int)},
     };
-    const int n_slots = (int)(sizeof slots / sizeof slots[0]), first_obs = 7;
+    const size_t first_obs = slots.size();
+    // ---- observation block (obs_begin .. obs_end)
+    if (flat) {
+      slots.push_back({(void**)&h->flat.base, N * A * D * f});
+    } else {
+      slots.insert(slots.end(), {
+        {(void**)&O.agent, N * A * Sw * f}, {(void**)&O.others, N * A * (A - 1) * Sw * f}, {(void**)&O.others_mask, N * A * (A - 1) * f},
+        {(void**)&O.zone, N * 6 * f}, {(void**)&O.heals, N * H * 2 * f}, {(void**)&O.heals_mask, N * A * H * f},
+        {(void**)&O.heal_slot, N * A * f}, {(void**)&O.heal_slot_mask, N * A * f}, {(void**)&O.boxes, N * B * 11 * f},
+        {(void**)&O.boxes_mask, N * A * B * f}, {(void**)&O.box_items, N * B * 10 * f}, {(void**)&O.box_items_mask, N * A * B * f},
+        {(void**)&O.box_slot, N * A * 8 * f}, {(void**)&O.box_slot_mask, N * A * f},
+        {(void**)&O.lidar_frac, N * A * L * f}});
+    }
+    slots.push_back({(void**)&O.lidar_hit, N * A * L * sizeof(int)});
     size_t off = 0; std::vector<size_t> offs;
-    for (int k = 0; k < n_slots; ++k) {
+    for (size_t k = 0; k < slots.size(); ++k) {
       if (k == first_obs) h->obs_begin = off;
       offs.push_back(off);
       off += (slots[k].bytes + 255) / 256 * 256;
     }
     h->obs_end = off; h->arena_bytes = off;
     rc |= dalloc(h, &h->arena, off);
-    if (!rc) for (int k = 0; k < n_slots; ++k) *slots[k].p = h->arena + offs[k];
+    if (!rc) for (size_t k = 0; k < slots.size(); ++k) *slots[k].p = h->arena + offs[k];
+    if (!rc && flat) O.lidar_frac = h->flat.base + (D - L);
   }
   rc |= dalloc(h, &S.obm, N); rc |= dalloc(h, &S.omask, AC * N);
   rc |= dalloc(h, &S.tq, N / (size_t)h->C.epb); rc |= dalloc(h, &S.tq_tail, 4);
@@ -477,6 +502,7 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
     std::vector<int> se(N, INT32_MIN);              // no reset record drawn yet
     cudaMemcpy(S.spare_ep, se.data(), N * sizeof(int), cudaMemcpyHostToDevice);
   }
+  int flat_col[MSV_OBS_KEYS] = {0};   // MSV_OBS_FLAT: first column of each key in an agent's row
   {  // the observation keys of k_obs2 (env:391-447 shapes)
     const int Ai = (int)A, Bi = (int)B, Hi = (int)H, Si = (int)Sw;
     ObsKey* K = h->obs.keys;
@@ -485,8 +511,28 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
     K[8] = {O.boxes, Bi * 11}; K[9] = {O.boxes_mask, Ai * Bi}; K[10] = {O.box_items, Bi * 10}; K[11] = {O.box_items_mask, Ai * Bi};
     K[12] = {O.box_slot, Ai * 8}; K[13] = {O.box_slot_mask, Ai};
     for (int k = 0; k < MSV_OBS_KEYS; ++k) if (obs_key_used(k, Hi, Bi)) h->obs_floats += K[k].chunk;
+    if (flat) {  // k_obs2's column map: where each column of an agent's row is in its stage (msv_types.cuh ObsFlat)
+      h->obs_floats = Ai * (int64_t)(D - L);
+      int koff[MSV_OBS_KEYS];
+      for (int k = 0, o = 0; k < MSV_OBS_KEYS; o += OBS2_E * K[k].chunk, ++k) koff[k] = o;
+      std::vector<int2> map(D, make_int2(0, 0));
+      int c = 0;
+      for (int k : kFlatOrder) {
+        if (!obs_key_used(k, Hi, Bi)) continue;
+        const bool shared = obs_key_shared(k);
+        const int w = shared ? K[k].chunk : K[k].chunk / Ai;
+        flat_col[k] = c;
+        for (int x = 0; x < w; ++x) map[c++] = make_int2(koff[k] + x, K[k].chunk | ((shared ? 0 : w) << 16));
+      }
+      int2* dmap = nullptr;
+      if (dalloc(h, &dmap, D) || cudaMemcpy(dmap, map.data(), D * sizeof(int2), cudaMemcpyHostToDevice) != cudaSuccess) {
+        g_err = h->err.empty() ? "cudaMemcpy(column map) failed" : h->err; msv_destroy(h); return MSV_ERR_ALLOC;
+      }
+      h->flat.map = dmap; h->flat.D = (int)D;
+      h->flat_term = h->flat; h->flat_term.base = nullptr;
+    }
     h->obs_term = h->obs;
-    if (cfg->auto_reset == 2) {
+    if (cfg->auto_reset == 2 && !flat) {
       for (int k = 0; k < MSV_OBS_KEYS; ++k) {
         float* buf = nullptr;
         if (dalloc(h, &buf, N * (size_t)(K[k].chunk > 0 ? K[k].chunk : 1))) { g_err = h->err; msv_destroy(h); return MSV_ERR_ALLOC; }
@@ -494,8 +540,12 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
       }
     }
     h->O_term = O;
+    if (cfg->auto_reset == 2 && flat) {
+      if (dalloc(h, &h->flat_term.base, N * A * D)) { g_err = h->err; msv_destroy(h); return MSV_ERR_ALLOC; }
+      h->O_term.lidar_frac = h->flat_term.base + (D - L);
+    }
     if (cfg->auto_reset == 2 && L > 0) {   // the finished episode's last scan, written by a second k_lidar
-      if (dalloc(h, &h->O_term.lidar_frac, N * A * L) || dalloc(h, &h->O_term.lidar_hit, N * A * L)) {
+      if ((!flat && dalloc(h, &h->O_term.lidar_frac, N * A * L)) || dalloc(h, &h->O_term.lidar_hit, N * A * L)) {
         g_err = h->err; msv_destroy(h); return MSV_ERR_ALLOC;
       }
     }
@@ -522,16 +572,28 @@ int msv_create(const msv_config* cfg, int32_t num_envs, int32_t device, uint64_t
   if (cfg->immunity_cooldown >= 0) reg(h, "immune", O.immune, 1, {n});
   if (cfg->battle_royale) { reg(h, "br_over", O.br_over, 1, {n}); reg(h, "br_results", O.br_results, 1, {n, a}); }
   if (cfg->max_episode_steps > 0) reg(h, "truncated", h->truncated, 1, {n});
-  if (cfg->auto_reset == 2) {   // same shapes, "terminal_" prefix
-    std::map<std::string, TensorInfo> extra;
-    static const char* names[MSV_OBS_KEYS] = {"agent", "others", "others_mask", "zone", "heals", "heals_mask", "heal_slot",
-                                              "heal_slot_mask", "boxes", "boxes_mask", "box_items", "box_items_mask", "box_slot", "box_slot_mask"};
+  if (flat) {   // the same names and shapes as views into obs_flat: a row of A*D floats per env, D per agent
+    const int64_t d = (int64_t)D;
+    reg(h, "obs_flat", h->flat.base, 0, {n, a, d});
     for (int k = 0; k < MSV_OBS_KEYS; ++k) {
-      auto it = h->tensors.find(names[k]);
+      auto it = h->tensors.find(kObsNames[k]);
       if (it == h->tensors.end()) continue;
-      TensorInfo t = it->second; t.ptr = h->obs_term.keys[k].base;
-      extra[std::string("terminal_") + names[k]] = t;
+      it->second.ptr = h->flat.base + flat_col[k];
+      it->second.strides[0] = a * d;
+      if (!obs_key_shared(k)) it->second.strides[1] = d;
     }
+    if (L > 0) { TensorInfo& t = h->tensors["lidar_frac"]; t.strides[0] = a * d; t.strides[1] = d; }
+  }
+  if (cfg->auto_reset == 2) {   // same shapes and strides, "terminal_" prefix
+    std::map<std::string, TensorInfo> extra;
+    for (int k = 0; k < MSV_OBS_KEYS; ++k) {
+      auto it = h->tensors.find(kObsNames[k]);
+      if (it == h->tensors.end()) continue;
+      TensorInfo t = it->second;
+      t.ptr = flat ? (void*)(h->flat_term.base + ((float*)t.ptr - h->flat.base)) : (void*)h->obs_term.keys[k].base;
+      extra[std::string("terminal_") + kObsNames[k]] = t;
+    }
+    if (flat) { extra["terminal_obs_flat"] = h->tensors["obs_flat"]; extra["terminal_obs_flat"].ptr = h->flat_term.base; }
     if (L > 0) {
       extra["terminal_lidar_frac"] = h->tensors["lidar_frac"]; extra["terminal_lidar_frac"].ptr = h->O_term.lidar_frac;
       extra["terminal_lidar_hit"] = h->tensors["lidar_hit"]; extra["terminal_lidar_hit"].ptr = h->O_term.lidar_hit;
@@ -664,9 +726,9 @@ static int launch(msv_handle* h, int which, const uint8_t* dev_in, void* stream)
       fin = h->finished;
     }
     if (h->cfg.auto_reset == 2) {
-      CK(msv_launch_obs(h->C, h->S, h->obs_term, h->AC, fin, st));
+      CK(msv_launch_obs(h->C, h->S, h->obs_term, h->flat.base ? &h->flat_term : nullptr, h->AC, fin, st));
       h->launches += 1;
-      if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O_term, h->BC, h->HC, st)); h->launches++; }
+      if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O_term, h->BC, h->HC, h->lidar_stride, st)); h->launches++; }
     }
     if (h->cfg.auto_reset != 0) {
       CK(msv_launch_reset(h->cap, h->C, h->S, h->O, fin, 1, nullptr, st));
@@ -683,11 +745,12 @@ static int launch(msv_handle* h, int which, const uint8_t* dev_in, void* stream)
     if (which == 0 && !handoff) { int rc = readback(h, st); if (rc) return rc; }
   }
   if (timed) tmark(h, st);
-  CK(msv_launch_obs(Cq, h->S, h->obs, h->AC, nullptr, st));   // fetch_observations
+  CK(msv_launch_obs(Cq, h->S, h->obs, h->flat.base ? &h->flat : nullptr, h->AC, nullptr, st));   // fetch_observations
   h->launches += 1;
   if (which == 0 && handoff) { int rc = readback(h, st); if (rc) return rc; }   // (an event between the two launches would serialise them)
   if (timed) tmark(h, st);
-  if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O, h->BC, h->HC, (cudaStream_t)stream)); h->launches++; }
+  // (every k_obs2 above is followed by its k_lidar: in the flat layout k_obs2 leaves the lidar columns to it)
+  if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O, h->BC, h->HC, h->lidar_stride, (cudaStream_t)stream)); h->launches++; }
   if (timed) tmark(h, st);
   const bool spare = which == 1 || (which == 0 && h->cfg.auto_reset != 0);
   if (spare) {                                  // the step / reset left finished environments without a record for their next episode
@@ -747,9 +810,10 @@ int msv_debug_step_kernel(msv_handle* h, const uint8_t* actions_dev, void* strea
   h->launches++;
   return MSV_OK;
 }
+// (k_obs2 alone: in the flat layout with lidars, the lidar columns it straddles are left as k_obs2 wrote them)
 int msv_debug_obs_kernel(msv_handle* h, void* stream) {
   if (!h) return MSV_ERR_INVALID;
-  CK(msv_launch_obs(h->C, h->S, h->obs, h->AC, nullptr, (cudaStream_t)stream));
+  CK(msv_launch_obs(h->C, h->S, h->obs, h->flat.base ? &h->flat : nullptr, h->AC, nullptr, (cudaStream_t)stream));
   h->launches++;
   return MSV_OK;
 }
@@ -776,7 +840,7 @@ int msv_render(msv_handle* h, int32_t first, int32_t count, int32_t height, int3
   DevGuard g(h->device);
   RenderArgs R = {};
   R.first = first; R.count = count; R.H = height; R.W = width; R.BC = h->BC; R.HC = h->HC;
-  R.lidar = (flags & MSV_RENDER_LIDAR) ? 1 : 0; R.out = out_dev;
+  R.lidar = (flags & MSV_RENDER_LIDAR) ? 1 : 0; R.LS = h->lidar_stride; R.out = out_dev;
   const cudaError_t e = msv_launch_render(h->C, h->S, h->O, R, (cudaStream_t)stream);
   h->launches++;
   h->last_was_step = false;    // the next k_step must not wait for an observation kernel that is not the last launch
@@ -893,8 +957,7 @@ int msv_tensor_info(msv_handle* h, const char* name, void** dev_ptr, int32_t* nd
   const TensorInfo& t = it->second;
   if (dev_ptr) *dev_ptr = t.ptr;
   if (ndim) *ndim = t.ndim;
-  int64_t st = 1;
-  for (int i = t.ndim - 1; i >= 0; --i) { if (shape) shape[i] = t.shape[i]; if (strides) strides[i] = st; st *= t.shape[i]; }
+  for (int i = 0; i < t.ndim; ++i) { if (shape) shape[i] = t.shape[i]; if (strides) strides[i] = t.strides[i]; }
   if (dtype_code) *dtype_code = t.dtype;
   return MSV_OK;
 }
@@ -918,8 +981,7 @@ int msv_tensor(msv_handle* h, const char* name, struct DLManagedTensor** out) {
   if (it == h->tensors.end()) { h->err = std::string("unknown tensor: ") + name; return MSV_ERR_NAME; }
   const TensorInfo& t = it->second;
   DLCtx* c = new DLCtx(); c->h = h;
-  int64_t st = 1;
-  for (int i = t.ndim - 1; i >= 0; --i) { c->shape[i] = t.shape[i]; c->strides[i] = st; st *= t.shape[i]; }
+  for (int i = 0; i < t.ndim; ++i) { c->shape[i] = t.shape[i]; c->strides[i] = t.strides[i]; }
   DLManagedTensor* m = new DLManagedTensor();
   m->dl_tensor.data = t.ptr;
   m->dl_tensor.device.device_type = 2;  // kDLCUDA

@@ -246,11 +246,16 @@ k_observe(const __grid_constant__ DevConst C, const __grid_constant__ DevState S
 // kRows (terminal capture): only the rows of real environments whose `only_if` byte is set are
 // written, with scalar stores (a row's slice of a key is not 16-byte aligned in general); the other
 // rows of the output are left untouched, and a tile without such a row leaves at once.
-#define OBS2_E 32
-template <bool kRows>
+// kFlat (MSV_OBS_FLAT): the stage keeps the layout above (a stage in the flat layout, with the keys stored once
+// per environment repeated for every agent, would not fit in shared memory for 8 agents); only the copy-out
+// changes.  The tile's rows of obs_flat are ONE contiguous run of rows * A * D floats, 16-byte aligned (e0 and
+// rows are multiples of 4), written with 16-byte stores, each float gathered from the stage through the
+// per-column map F.map (held in shared memory after the stage).  A float4 that holds only lidar columns is not
+// written (k_lidar writes them after this kernel); one that straddles them writes stage[0] there.
+template <bool kRows, bool kFlat>
 __global__ void __launch_bounds__(1024)
 k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, const __grid_constant__ ObsTable Tb, int AC,
-       const uint8_t* __restrict__ only_if) {
+       const uint8_t* __restrict__ only_if, const ObsFlat F) {
   extern __shared__ float stage[];
   const int A = C.A, B = C.B0, H = C.H0, Sw = C.S, N = C.N;
   // A tile is (part of) the environments of one k_step block: block `kb`, sub-tile `sub` of up to OBS2_E rows.
@@ -287,11 +292,12 @@ k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, c
   const int e0 = kb * C.epb + sub * OBS2_E, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   int rows = C.epb - sub * OBS2_E; if (rows > OBS2_E) rows = OBS2_E;   // a multiple of 32 / G >= 4: every run below is a whole number of float4
   // this lane's row of every tensor slice in the stage (registers: the key is a compile-time constant at every use)
-  int koff[MSV_OBS_KEYS], kbase[MSV_OBS_KEYS];
+  int koff[MSV_OBS_KEYS], kbase[MSV_OBS_KEYS], stage_floats = 0;
   {
     int o = 0;
 #pragma unroll
     for (int k = 0; k < MSV_OBS_KEYS; ++k) { koff[k] = o; kbase[k] = o + lane * Tb.keys[k].chunk; o += OBS2_E * Tb.keys[k].chunk; }
+    stage_floats = o;
   }
   const int e = e0 + lane;
   const bool live = lane < rows;                 // (e < N: the padded batch is a whole number of k_step blocks)
@@ -300,6 +306,9 @@ k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, c
     sel = __ballot_sync(0xffffffffu, live && e < C.n_real && only_if[e] != 0);
     if (!sel) return;
   }
+  int2* fmap = reinterpret_cast<int2*>(stage + stage_floats);
+  if (kFlat)
+    for (int c = threadIdx.x; c < F.D; c += blockDim.x) fmap[c] = __ldg(&F.map[c]);
   const int n_items = A + 2 * B + H + 1;
   // (state loads below bypass L1 -- __ldcg: each word is read once, and with the hand-off on it was written by a
   // block of the still-running step kernel on another SM)
@@ -389,19 +398,45 @@ k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, c
   }
   __syncthreads();
   TRACE(5, blockIdx.x);
-  for (int k = 0; k < MSV_OBS_KEYS; ++k) {
-    const int chunk = Tb.keys[k].chunk;
-    if (chunk <= 0 || !obs_key_used(k, H, B)) continue;
+  if (kFlat) {
+    const int D = F.D, AD = A * D, DL = D - C.lidar_n;
+    float* dst = F.base + (size_t)e0 * AD;
+    auto gather = [&](int r, int i, int c) { const int2 m = fmap[c]; return stage[m.x + r * (m.y & 0xffff) + i * (m.y >> 16)]; };
     if (kRows) {
-      const float* src = stage + koff[k];
-      float* dst = Tb.keys[k].base + (size_t)e0 * chunk;
-      for (int q = threadIdx.x; q < rows * chunk; q += blockDim.x)
-        if ((sel >> (q / chunk)) & 1u) dst[q] = src[q];
+      for (int q = threadIdx.x; q < rows * AD; q += blockDim.x) {
+        const int r = q / AD, rem = q - r * AD, i = rem / D, c = rem - i * D;
+        if (((sel >> r) & 1u) && c < DL) dst[q] = gather(r, i, c);
+      }
     } else {
-      const int n4 = rows * chunk / 4;
-      const float4* src = reinterpret_cast<const float4*>(stage + koff[k]);
-      float4* dst = reinterpret_cast<float4*>(Tb.keys[k].base + (size_t)e0 * chunk);
-      for (int q = threadIdx.x; q < n4; q += blockDim.x) dst[q] = src[q];
+      float4* dst4 = reinterpret_cast<float4*>(dst);
+      for (int q4 = threadIdx.x; q4 < rows * AD / 4; q4 += blockDim.x) {
+        const int q = 4 * q4;
+        int r = q / AD; const int rem = q - r * AD; int i = rem / D; int c = rem - i * D;
+        if (c >= DL && c + 3 < D) continue;      // four lidar columns of one agent's row
+        float v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          v[u] = gather(r, i, c);
+          if (++c == D) { c = 0; if (++i == A) { i = 0; ++r; } }
+        }
+        dst4[q4] = make_float4(v[0], v[1], v[2], v[3]);
+      }
+    }
+  } else {
+    for (int k = 0; k < MSV_OBS_KEYS; ++k) {
+      const int chunk = Tb.keys[k].chunk;
+      if (chunk <= 0 || !obs_key_used(k, H, B)) continue;
+      if (kRows) {
+        const float* src = stage + koff[k];
+        float* dst = Tb.keys[k].base + (size_t)e0 * chunk;
+        for (int q = threadIdx.x; q < rows * chunk; q += blockDim.x)
+          if ((sel >> (q / chunk)) & 1u) dst[q] = src[q];
+      } else {
+        const int n4 = rows * chunk / 4;
+        const float4* src = reinterpret_cast<const float4*>(stage + koff[k]);
+        float4* dst = reinterpret_cast<float4*>(Tb.keys[k].base + (size_t)e0 * chunk);
+        for (int q = threadIdx.x; q < n4; q += blockDim.x) dst[q] = src[q];
+      }
     }
   }
   TRACE(4, blockIdx.x);
@@ -427,7 +462,8 @@ k_obs2(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, c
 #define LID_MAXB 64            // >= MSV_MAX_BOXES * 2 + MSV_MAX_HEALS + 4 + MSV_MAX_AGENTS = 44
 #define LID_W 9
 __global__ void __launch_bounds__(256)
-k_lidar(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, const __grid_constant__ DevOut O, int EB, int BC, int HC) {
+k_lidar(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, const __grid_constant__ DevOut O, int EB, int BC, int HC,
+        int LS) {
   extern __shared__ float lid_sm[];                  // [EB][LID_MAXB][LID_W]: kind, x, y, then r | hx, hy, ax, ay, rot (agents: r, angle); [8] body seq
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // (the next step's k_step may be waiting to become resident)
   const int A = C.A, L = C.lidar_n, N = C.N;
@@ -472,9 +508,9 @@ k_lidar(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, 
   if (!on) return;
   const float* mine = tab + (oA + i) * LID_W;
   const bool alive_i = __float_as_int(mine[0]) == KIND_AGENT;
-  const size_t obase = ((size_t)e * A + i) * L;
+  const size_t obase = ((size_t)e * A + i) * L, fbase = ((size_t)e * A + i) * LS;   // lidar_frac rows: LS apart (flat layout: D)
   if (!alive_i) {                                    // dead agents have no Lidars row: reported as "no hit"
-    if (lane < L) { O.lidar_frac[obase + lane] = 1.0f; O.lidar_hit[obase + lane] = 0; }
+    if (lane < L) { O.lidar_frac[fbase + lane] = 1.0f; O.lidar_hit[obase + lane] = 0; }
     return;
   }
   const f2 me = mk2(mine[1], mine[2]);
@@ -560,7 +596,7 @@ k_lidar(const __grid_constant__ DevConst C, const __grid_constant__ DevState S, 
       else { kind = KIND_AGENT; idx = bestb - oA; }
       hitcode = (kind << 8) | idx;
     }
-    O.lidar_frac[obase + r] = fr;
+    O.lidar_frac[fbase + r] = fr;
     O.lidar_hit[obase + r] = hitcode;
   }
 }
@@ -618,13 +654,13 @@ __global__ void k_stats(int N, int stride, int AC, float* sreward, int* skills, 
 }
 
 // ------------------------------------------------------------- launchers ---
-template <bool kRows>
+template <bool kRows, bool kFlat>
 static cudaError_t obs_attrs() {
   // the stage of the 8-agent class is ~1 000 floats x 32 environments, far over the 48 KB default
-  cudaError_t e = cudaFuncSetAttribute(k_obs2<kRows>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  cudaError_t e = cudaFuncSetAttribute(k_obs2<kRows, kFlat>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
   // same L1/shared split as the step kernel, so that a tile can become resident on an SM that still runs one of its blocks
   if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_obs2<kRows>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    e = cudaFuncSetAttribute(k_obs2<kRows, kFlat>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   return e;
 }
 
@@ -640,8 +676,10 @@ static cudaError_t launch_t(int which, const DevConst& C, const DevState& S, con
     cudaError_t e = cudaFuncSetAttribute(k_step<AC, BC, HC, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_reset<AC, BC, HC, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_observe<AC, BC, HC, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
-    if (e == cudaSuccess) e = obs_attrs<false>();
-    if (e == cudaSuccess) e = obs_attrs<true>();
+    if (e == cudaSuccess) e = obs_attrs<false, false>();
+    if (e == cudaSuccess) e = obs_attrs<true, false>();
+    if (e == cudaSuccess) e = obs_attrs<false, true>();
+    if (e == cudaSuccess) e = obs_attrs<true, true>();
     return e;
   }
   if (which == 0 && C.pdl_wait) {
@@ -690,9 +728,11 @@ cudaError_t msv_launch_truncate(const DevConst& C, const DevState& S, const DevO
   return cudaPeekAtLastError();
 }
 
-cudaError_t msv_launch_obs(const DevConst& C, const DevState& S, const ObsTable& T, int AC, const uint8_t* only_if, cudaStream_t st) {
+cudaError_t msv_launch_obs(const DevConst& C, const DevState& S, const ObsTable& T, const ObsFlat* F, int AC, const uint8_t* only_if,
+                           cudaStream_t st) {
   size_t smem = 0;
   for (int k = 0; k < MSV_OBS_KEYS; ++k) smem += (size_t)OBS2_E * T.keys[k].chunk * sizeof(float);
+  if (F) smem += (size_t)F->D * sizeof(int2);                          // the column map
   // one warp per source item when they fit a block (a single round of loads), else 32 warps looping over the items
   const int n_items = C.A + 2 * C.B0 + C.H0 + 1;
   const int threads = n_items <= 32 ? 32 * n_items : 1024;
@@ -704,15 +744,18 @@ cudaError_t msv_launch_obs(const DevConst& C, const DevState& S, const ObsTable&
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;                // may start before the step kernel has finished
   cfg.attrs = at; cfg.numAttrs = C.tq_ticket ? 1 : 0;
-  if (only_if) return cudaLaunchKernelEx(&cfg, k_obs2<true>, C, S, T, AC, only_if);
-  return cudaLaunchKernelEx(&cfg, k_obs2<false>, C, S, T, AC, only_if);
+  const ObsFlat none = {nullptr, nullptr, 0};
+  if (F && only_if) return cudaLaunchKernelEx(&cfg, k_obs2<true, true>, C, S, T, AC, only_if, *F);
+  if (F) return cudaLaunchKernelEx(&cfg, k_obs2<false, true>, C, S, T, AC, only_if, *F);
+  if (only_if) return cudaLaunchKernelEx(&cfg, k_obs2<true, false>, C, S, T, AC, only_if, none);
+  return cudaLaunchKernelEx(&cfg, k_obs2<false, false>, C, S, T, AC, only_if, none);
 }
 
-cudaError_t msv_launch_lidar(const DevConst& C, const DevState& S, const DevOut& O, int BC, int HC, cudaStream_t st) {
+cudaError_t msv_launch_lidar(const DevConst& C, const DevState& S, const DevOut& O, int BC, int HC, int LS, cudaStream_t st) {
   int EB = 8 / C.A; if (EB < 1) EB = 1;              // whole environments per block, 8 warps (A = 8: one env; A = 4: two; A <= 2: four)
   const int warps = EB * C.A;
   const size_t smem = (size_t)EB * LID_MAXB * LID_W * sizeof(float);
-  k_lidar<<<(C.n_real + EB - 1) / EB, warps * 32, smem, st>>>(C, S, O, EB, BC, HC);
+  k_lidar<<<(C.n_real + EB - 1) / EB, warps * 32, smem, st>>>(C, S, O, EB, BC, HC, LS);
   return cudaPeekAtLastError();
 }
 

@@ -22,13 +22,17 @@ cudaError_t msv_read_blocks(unsigned long long* out, int n_words);
 cudaError_t msv_read_trace(unsigned long long* out, int n_words);
 cudaError_t msv_read_check(unsigned long long out[2]);
 cudaError_t msv_launch_spare(const DevConst& C, const DevState& S, const uint8_t* dones, int only_done, cudaStream_t st);
-// k_obs2 into T's tensors: every row (only_if NULL), or the rows of the real envs whose only_if byte is set
-cudaError_t msv_launch_obs(const DevConst& C, const DevState& S, const ObsTable& T, int AC, const uint8_t* only_if, cudaStream_t st);
-cudaError_t msv_launch_lidar(const DevConst& C, const DevState& S, const DevOut& O, int BC, int HC, cudaStream_t st);
+// k_obs2 into T's tensors (F NULL) or into F's flat rows: every row (only_if NULL), or the rows of the real envs
+// whose only_if byte is set
+cudaError_t msv_launch_obs(const DevConst& C, const DevState& S, const ObsTable& T, const ObsFlat* F, int AC, const uint8_t* only_if,
+                           cudaStream_t st);
+// k_lidar; LS: floats between two agents' rows of O.lidar_frac (L in the dict layout, D in the flat one)
+cudaError_t msv_launch_lidar(const DevConst& C, const DevState& S, const DevOut& O, int BC, int HC, int LS, cudaStream_t st);
 // msv_render: picture of envs [first, first+count) into out (uint8[count][H][W][3]); BC, HC the list capacities,
-// lidar != 0 draws the rays.  The launcher fills in the tiling and the viewport (the fields after `lidar`).
+// lidar != 0 draws the rays (LS: the row stride of O.lidar_frac, as k_lidar).  The launcher fills in the tiling
+// and the viewport (the fields after `LS`).
 struct RenderArgs {
-  int first, count, H, W, BC, HC, lidar;
+  int first, count, H, W, BC, HC, lidar, LS;
   int TW, TR, tiles_x, tiles_per_img;   // tile width and rows, tiles per image row and per image
   float s, half_floor;                  // pixel size, floor_size / 2
   uint8_t* out;

@@ -161,7 +161,7 @@ k_render(const __grid_constant__ DevConst C, const __grid_constant__ DevState S,
           keep = (__float_as_int(S.akin1[i * N + e].w) & 1) != 0;
           float ex, ey, w;
           if (ray) {                                     // k_lidar: off = from_polar(depth, (float)(ang + heading))
-            const float frac = O.lidar_frac[((size_t)e * A + i) * L + r];
+            const float frac = O.lidar_frac[((size_t)e * A + i) * R.LS + r];
             float sn, cs; rnd_sincos((float)(C.lidar_ang[r] + (double)k0.z), sn, cs);
             const float L0 = C.lidar_depth;
             const float offx = cs * L0 + (-sn) * 0.0f, offy = sn * L0 + cs * 0.0f;

@@ -125,7 +125,14 @@ struct DevOut {
 // ---- observation writer (k_obs2) -----------------------------------------
 // The observation keys in DevOut order (agent .. box_slot_mask): tensor base and floats per environment.
 struct ObsKey { float* base; int chunk; };
+#define OBS2_E 32   // environments per k_obs2 tile: the stage holds key k of the tile at OBS2_E * (chunks of the keys before k)
 #define MSV_OBS_KEYS 14
 struct ObsTable { ObsKey keys[MSV_OBS_KEYS]; };
 // keys 4-7 (heals ..) exist only with heals, keys 8-13 (boxes ..) only with boxes
 __host__ __device__ inline bool obs_key_used(int k, int H, int B) { return !((k >= 4 && k <= 7 && H == 0) || (k >= 8 && B == 0)); }
+// MSV_OBS_FLAT: k_obs2 writes rows [e][i] of D floats into `base` ([N][A][D]).  map[c] (D entries) says where
+// column c of agent i in environment row r of the tile is in the stage: stage[x + r * (y & 0xffff) + i * (y >> 16)],
+// i.e. x = the float's offset for row 0 and agent 0, then the key's floats per environment and per agent (0 for
+// the keys stored once per environment).  The last L columns are lidar_frac, written by k_lidar after k_obs2 in
+// every sequence that runs k_obs2: their entries are {0, 0}.
+struct ObsFlat { float* base; const int2* map; int D; };

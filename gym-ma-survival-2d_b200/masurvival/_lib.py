@@ -108,7 +108,7 @@ def load():
     L.msv_debug_overflow.restype = i64
     L.msv_debug_check_failures.argtypes = [vp, ctypes.POINTER(i64)]
     L.msv_debug_check_failures.restype = i64
-    if L.msv_abi_version() != 2:
+    if L.msv_abi_version() != 3:
         raise MasurvError('libmasurv.so ABI version mismatch')
     for name, dt in (('msv_sizeof_config', CONFIG_DT), ('msv_sizeof_env_state', STATE_DT),
                      ('msv_sizeof_stats', STATS_DT)):
@@ -166,6 +166,15 @@ class Handle:
             cap = _PyCapsule_New(m, b'dltensor', None)
             self._tensors[name] = torch.from_dlpack(cap)
         return self._tensors[name]
+
+    def tensor_info(self, name):
+        """msv_tensor_info: (device pointer, shape, strides in elements, dtype code 0 f32 / 1 u8 / 2 i32)"""
+        p, nd, dt = ctypes.c_void_p(), ctypes.c_int32(), ctypes.c_int32()
+        shape, strides = (ctypes.c_int64 * 4)(), (ctypes.c_int64 * 4)()
+        check(load().msv_tensor_info(self.h, name.encode(), ctypes.byref(p), ctypes.byref(nd), shape, strides,
+                                     ctypes.byref(dt)), self.h)
+        n = nd.value
+        return p.value or 0, tuple(shape[:n]), tuple(strides[:n]), dt.value
 
     def has_tensor(self, name):
         p = ctypes.c_void_p()

@@ -108,9 +108,16 @@ def _radius(shape):
     return float(shape)
 
 
-def pack_config(cfg, continuous_melee=False, auto_reset=False, max_episode_steps=0):
+OBS_LAYOUTS = ('dict', 'flat')    # msv_config.obs_layout: MSV_OBS_DICT, MSV_OBS_FLAT
+
+
+def pack_config(cfg, continuous_melee=False, auto_reset=False, max_episode_steps=0, obs_layout='dict'):
     """Nested (merged) config dict -> msv_config record (numpy void).  `max_episode_steps`: the
-    step limit of the vector env (0 = none), an extension the reference does not have."""
+    step limit of the vector env (0 = none), an extension the reference does not have.
+    `obs_layout`: 'dict' (one tensor per observation key) or 'flat' (one [N, A, D] tensor, the keys
+    as views into it; see MaSurvivalVec.flat_obs)."""
+    if obs_layout not in OBS_LAYOUTS:
+        raise ValueError(f"obs_layout must be 'dict' or 'flat', not {obs_layout!r}")
     rec = np.zeros((), dtype=CONFIG_DT)
     agents = cfg['agents']
     rec['n_agents'] = agents.get('n_spawns', agents.get('n_agents'))
@@ -183,6 +190,7 @@ def pack_config(cfg, continuous_melee=False, auto_reset=False, max_episode_steps
     # False/0 off, True/1 in-kernel reset, 'terminal'/2 reset + terminal observation capture
     rec['auto_reset'] = 2 if auto_reset in ('terminal', 2) else int(bool(auto_reset))
     rec['max_episode_steps'] = int(max_episode_steps)
+    rec['obs_layout'] = OBS_LAYOUTS.index(obs_layout)
     validate(rec)
     return rec
 

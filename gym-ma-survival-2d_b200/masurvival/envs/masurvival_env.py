@@ -43,14 +43,22 @@ class MaSurvivalVec:
                             episode_length rows are valid where done | truncated,
                             and auto_reset treats it like a finished episode
                             (auto_reset=False only flags it: see reset_envs)
+    obs_layout : str        'dict' (default): the library writes one tensor per
+                            observation key.  'flat': it writes one float32
+                            tensor [N, A, D], one row per agent (flat_obs(),
+                            flat_obs_layout()), ready for a policy shared by
+                            the agents; the observation dicts are the same,
+                            as strided views into it
     """
 
     metadata = {'render_modes': ['rgb_array'], 'render_fps': 30}
 
-    def __init__(self, config=None, num_envs=1, device=0, seed=0, env_offset=0, auto_reset=True, max_episode_steps=None):
+    def __init__(self, config=None, num_envs=1, device=0, seed=0, env_offset=0, auto_reset=True, max_episode_steps=None,
+                 obs_layout='dict'):
         self.config, self._continuous_melee = merge_config(config)
         self._rec = pack_config(self.config, self._continuous_melee, auto_reset=auto_reset,
-                                max_episode_steps=max_episode_steps or 0)
+                                max_episode_steps=max_episode_steps or 0, obs_layout=obs_layout)
+        self.obs_layout = obs_layout
         self.num_envs = int(num_envs)
         self.device = int(device)
         self.auto_reset = bool(auto_reset)
@@ -131,6 +139,24 @@ class MaSurvivalVec:
             x[k] = t
         return x
 
+    def flat_obs(self):
+        """obs_layout='flat': the float32 tensor [N, A, D] the library writes, row [e, i] = agent i's
+        observation: obs[k][e, i].ravel() concatenated over the keys of obs_shapes() in their order,
+        lidar_hit excepted (column ranges: flat_obs_layout()).  Zero-copy, the same storage on every
+        call; like every output it is valid until the next step / reset / observe."""
+        if self.obs_layout != 'flat':
+            raise RuntimeError("flat_obs() needs MaSurvivalVec(..., obs_layout='flat')")
+        return self._h.tensor('obs_flat')
+
+    def flat_obs_layout(self):
+        """obs_layout='flat': {key: (first column, per-agent shape)} in column order (the order of
+        obs_shapes()), the columns read from the library's tensor pointers."""
+        if self.obs_layout != 'flat':
+            raise RuntimeError("flat_obs_layout() needs MaSurvivalVec(..., obs_layout='flat')")
+        base = self._h.tensor_info('obs_flat')[0]
+        return {k: ((self._h.tensor_info(k)[0] - base) // 4, shp[1:])
+                for k, shp in self.obs_shapes().items() if k != 'lidar_hit'}
+
     def _stream(self):
         import torch
         return torch.cuda.current_stream(self.device).cuda_stream
@@ -206,6 +232,8 @@ class MaSurvivalVec:
         self._h.step(a.data_ptr(), self._stream())
         self.steps += 1
         info = {'terminal_observation': self._obs('terminal_')} if self._terminal else {}
+        if self._terminal and self.obs_layout == 'flat':
+            info['terminal_observation_flat'] = self._h.tensor('terminal_obs_flat')
         # per-env episode statistics (rows valid where done, or done | truncated under a step limit): what a
         # trainer logs at episode end
         info['episode_return'] = self._h.tensor('episode_return')
@@ -264,21 +292,24 @@ class MaSurvivalVec:
     def host_obs_buffer(self, pinned=True):
         """A host buffer for step_host_obs (page-locked by default) and the dict of
         zero-copy numpy views into it, one per observation key (library layout:
-        `zone/heals/boxes/box_items` once per env, see _obs)."""
+        `zone/heals/boxes/box_items` once per env, see _obs; with obs_layout='flat'
+        strided views into the flat rows)."""
         import torch
         nbytes = self._h.obs_host_bytes()
         buf = torch.empty(nbytes, dtype=torch.uint8)
         if pinned:
             buf = buf.pin_memory()
         raw = buf.numpy()
-        views, N, A = {}, self.num_envs, self.n_agents
-        for k, shp in self.obs_shapes().items():
+        views = {}
+        for k in self.obs_shapes():
             off = self._h.obs_host_offset(k)
-            if k in ('zone', 'heals', 'boxes', 'box_items'):
-                shp = shp[1:]
+            _, shape, strides, _ = self._h.tensor_info(k)
             dt = np.int32 if k == 'lidar_hit' else np.float32
-            n = int(np.prod(shp)) * N
-            views[k] = raw[off:off + 4 * n].view(dt).reshape((N,) + tuple(shp))
+            if self.obs_layout == 'flat':
+                views[k] = np.lib.stride_tricks.as_strided(raw[off:].view(dt), shape, tuple(4 * s for s in strides))
+            else:
+                n = int(np.prod(shape))
+                views[k] = raw[off:off + 4 * n].view(dt).reshape(shape)
         return buf, views
 
     def step_host_obs(self, actions, obs_buf, rewards_out=None, dones_out=None):

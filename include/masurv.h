@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MSV_ABI_VERSION 2
+#define MSV_ABI_VERSION 3
 
 /* Compile-time capacities (per environment). */
 #define MSV_MAX_AGENTS 8
@@ -123,7 +123,18 @@ typedef struct msv_config {
    * (and auto_reset 2 keeps their last observation), auto_reset 0 only flags them (msv_reset_envs).
    * The observation hand-off is off (msv_tile_plan out[3] = 0).  Negative values are refused. */
   int32_t max_episode_steps;
+  /* Layout of the observation outputs: MSV_OBS_DICT writes one tensor per key; MSV_OBS_FLAT writes one
+   * float32 tensor "obs_flat" [num_envs][n_agents][D] whose row [e][i] is agent i's observation: the
+   * concatenation, in the order agent, zone, others, others_mask, heals, heals_mask, heal_slot,
+   * heal_slot_mask, boxes, boxes_mask, box_items, box_items_mask, box_slot, box_slot_mask, lidar_frac,
+   * of every key the config has (the keys stored once per env repeated in every agent's row).  Every key
+   * keeps its name and dict-mode shape as a strided view into it (msv_tensor_info reports the strides);
+   * "lidar_hit" stays a tensor of its own.  Other values are refused. */
+  int32_t obs_layout;
+  int32_t reserved1;       /* must be 0 */
 } msv_config;
+#define MSV_OBS_DICT 0
+#define MSV_OBS_FLAT 1
 #define MSV_B2_CLAMP_DAMPING 1
 #define MSV_B2_WELD_SQUARED 2
 #define MSV_B2_SUBSTEPS_GE 4
@@ -280,8 +291,9 @@ int msv_step_host(msv_handle* h, const uint8_t* actions_host,
 /* The same step returning the OBSERVATIONS as well (env:84,90: the step's main
  * result).  obs_host receives msv_obs_host_bytes() bytes: every observation
  * tensor (and the lidar block) in the library's de-duplicated layout, tensor
- * `name` at byte offset msv_obs_host_offset(name), row-major with the shape
- * msv_tensor_info reports.  One device->host copy on the internal stream after
+ * `name` at byte offset msv_obs_host_offset(name) (its first element), with the
+ * shape and strides msv_tensor_info reports (MSV_OBS_FLAT: the block is
+ * [obs_flat | lidar_hit] and the keys are strided views into obs_flat).  One device->host copy on the internal stream after
  * the observation kernels. */
 int msv_step_host_obs(msv_handle* h, const uint8_t* actions_host,
                       float* rewards_host, uint8_t* dones_host, void* obs_host,
@@ -308,11 +320,13 @@ int64_t msv_obs_host_offset(msv_handle* h, const char* name); /* -1: unknown */
  * "episode_return", "episode_length", "lidar_frac", "lidar_hit", and
  * "truncated" (uint8[num_envs], only with max_episode_steps > 0: 1 where the
  * step limit ended the episode on the last step and the game did not; the
- * episode_* rows are valid where dones | truncated).  The deleter only drops
- * a refcount. */
+ * episode_* rows are valid where dones | truncated).  With MSV_OBS_FLAT also
+ * "obs_flat" (and "terminal_obs_flat" under auto_reset 2); the observation
+ * keys are then strided views into it (the strides are part of the export).
+ * The deleter only drops a refcount. */
 int msv_tensor(msv_handle* h, const char* name, struct DLManagedTensor** out);
 
-/* Raw view of the same tensors (for non-DLPack callers / tests). */
+/* Raw view of the same tensors (for non-DLPack callers / tests); strides in elements. */
 int msv_tensor_info(msv_handle* h, const char* name, void** dev_ptr,
                     int32_t* ndim, int64_t shape[4], int64_t strides[4],
                     int32_t* dtype_code /*0 f32, 1 u8, 2 i32*/);
