@@ -70,6 +70,9 @@ struct msv_handle {
   int lidar_stride = 0;      // floats between two agents' rows of lidar_frac: L (dict) or D (flat)
   uint8_t* truncated = nullptr;   // max_episode_steps > 0: the "truncated" tensor [N]
   uint8_t* finished = nullptr;    // max_episode_steps > 0: dones | truncated of the last step [N] (k_truncate)
+  // msv_enable_global_state: k_global_state writes "global_state" (and, auto_reset 2, "terminal_global_state"),
+  // [N][gs.Ds] floats each, after the observation kernels of every call that writes observations
+  bool gs_on = false; GsLayout gs = {}; float* gs_buf = nullptr; float* gs_term = nullptr;
   int64_t exported;          // live DLPack exports
   std::string err;
 };
@@ -729,6 +732,7 @@ static int launch(msv_handle* h, int which, const uint8_t* dev_in, void* stream)
       CK(msv_launch_obs(h->C, h->S, h->obs_term, h->flat.base ? &h->flat_term : nullptr, h->AC, fin, st));
       h->launches += 1;
       if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O_term, h->BC, h->HC, h->lidar_stride, st)); h->launches++; }
+      if (h->gs_on) { CK(msv_launch_global_state(h->C, h->S, h->gs, h->gs_term, fin, st)); h->launches++; }
     }
     if (h->cfg.auto_reset != 0) {
       CK(msv_launch_reset(h->cap, h->C, h->S, h->O, fin, 1, nullptr, st));
@@ -752,6 +756,9 @@ static int launch(msv_handle* h, int which, const uint8_t* dev_in, void* stream)
   // (every k_obs2 above is followed by its k_lidar: in the flat layout k_obs2 leaves the lidar columns to it)
   if (h->C.lidar_n > 0) { CK(msv_launch_lidar(h->C, h->S, h->O, h->BC, h->HC, h->lidar_stride, (cudaStream_t)stream)); h->launches++; }
   if (timed) tmark(h, st);
+  // the global state describes the same state as the observations (a plain launch: the next k_step may be
+  // programmatically dependent on it, as on k_lidar)
+  if (h->gs_on) { CK(msv_launch_global_state(h->C, h->S, h->gs, h->gs_buf, nullptr, st)); h->launches++; }
   const bool spare = which == 1 || (which == 0 && h->cfg.auto_reset != 0);
   if (spare) {                                  // the step / reset left finished environments without a record for their next episode
     if (!h->side_stream) {
@@ -827,6 +834,60 @@ int msv_observe(msv_handle* h, void* stream) { return h ? launch(h, 2, nullptr, 
 int msv_step(msv_handle* h, const uint8_t* actions_dev, void* stream) {
   if (!h || !actions_dev) return MSV_ERR_INVALID;
   return launch(h, 0, actions_dev, stream);
+}
+
+// the "global_state" row of an env of cfg (gs_layout), with a view "global_state_<key>" per key
+static const char* const kGsNames[GS_KEYS] = {"agents", "agents_mask", "zone", "heals", "heals_mask", "heal_slot", "heal_slot_mask",
+                                               "boxes", "boxes_mask", "box_items", "box_items_mask", "box_slot", "box_slot_mask", "steps"};
+
+int msv_global_state_dim(const msv_config* cfg) {
+  if (!cfg || cfg->n_agents < 1 || cfg->n_agents > MSV_MAX_AGENTS || cfg->n_boxes < 0 || cfg->n_boxes > MSV_MAX_BOXES ||
+      cfg->n_heals < 0 || cfg->n_heals > MSV_MAX_HEALS)
+    return MSV_ERR_INVALID;
+  return gs_layout(cfg->n_agents, cfg->n_boxes, cfg->n_heals, 8 + (cfg->teams ? 1 : 0)).Ds;
+}
+
+int msv_enable_global_state(msv_handle* h, void* stream) {
+  if (!h) return MSV_ERR_INVALID;
+  DevGuard g(h->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone) {
+    h->err = "msv_enable_global_state: the stream is being captured (the call allocates)";
+    return MSV_ERR_INVALID;
+  }
+  if (!h->gs_on) {
+    const msv_config& c = h->cfg;
+    const GsLayout Lg = gs_layout(c.n_agents, c.n_boxes, c.n_heals, h->C.S);
+    const size_t N = (size_t)h->C.N;
+    CK(msv_global_state_attrs());                 // on the handle's device (the DevGuard above)
+    if (dalloc(h, &h->gs_buf, N * Lg.Ds)) return MSV_ERR_ALLOC;
+    if (c.auto_reset == 2) {                      // rows not finished on a step keep their bytes: start from zeros in stream order
+      if (dalloc(h, &h->gs_term, N * Lg.Ds)) return MSV_ERR_ALLOC;
+      CK(cudaMemsetAsync(h->gs_term, 0, N * Lg.Ds * sizeof(float), st));
+    }
+    const int64_t n = h->C.n_real, a = c.n_agents, b = c.n_boxes, hh = c.n_heals, s = h->C.S, d = Lg.Ds;
+    const std::vector<std::vector<int64_t>> shapes = {{a, s}, {a}, {6}, {hh, 2}, {hh}, {a}, {a}, {b, 11}, {b}, {b, 10}, {b}, {a, 8}, {a}, {1}};
+    auto add = [&](const std::string& prefix, float* base) {
+      TensorInfo t = {}; t.ptr = base; t.ndim = 2; t.dtype = 0; t.shape[0] = n; t.shape[1] = d; t.strides[0] = d; t.strides[1] = 1;
+      h->tensors[prefix] = t;
+      for (int k = 0; k < GS_KEYS; ++k) {
+        if ((k >= GS_HEALS && k <= GS_HEAL_SLOT_MASK && hh == 0) || (k >= GS_BOXES && k <= GS_BOX_SLOT_MASK && b == 0)) continue;
+        TensorInfo v = {}; v.ptr = base + Lg.col[k]; v.dtype = 0; v.ndim = 1 + (int)shapes[k].size();
+        v.shape[0] = n; v.strides[0] = d;
+        int64_t st_ = 1;
+        for (int i = v.ndim - 1; i >= 1; --i) { v.shape[i] = shapes[k][i - 1]; v.strides[i] = st_; st_ *= v.shape[i]; }
+        h->tensors[prefix + "_" + kGsNames[k]] = v;
+      }
+    };
+    add("global_state", h->gs_buf);
+    if (h->gs_term) add("terminal_global_state", h->gs_term);
+    h->gs = Lg; h->gs_on = true;
+  }
+  CK(msv_launch_global_state(h->C, h->S, h->gs, h->gs_buf, nullptr, st));
+  h->launches++;
+  h->last_was_step = false;    // the next k_step must not wait programmatically on a kernel that is not an observation kernel of a step
+  return MSV_OK;
 }
 
 int msv_render(msv_handle* h, int32_t first, int32_t count, int32_t height, int32_t width, uint32_t flags,
@@ -1169,6 +1230,9 @@ int msv_flush_stats(msv_handle* h, msv_stats* out) {
 //   which 1: k_obs2   reads  agents (akin0, akin1, aint) 48*A, obm 8 (+ omask 4*A), hdr0 16, boxes 32*B, items 16*B,
 //                            heals 8*H, zone 32 + next centre 8;   writes the observation tensors
 //   which 2: k_lidar  reads  hdr0 16, boxes 32*B, items 16*B, heals 8*H, agents (akin0, akin1) 32*A;  writes 8*A*L
+//   which 3: k_global_state (only once msv_enable_global_state was called)
+//                     reads  agents (akin0, akin1, aint) 48*A, hdr0 16, boxes 32*B, items 16*B, heals 8*H, zone 32 + next
+//                            centre 8;   writes the row, 4*Ds
 int64_t msv_kernel_bytes_per_env(msv_handle* h, int32_t which) {
   if (!h) return 0;
   const int64_t A = h->C.A, B = h->C.B0, H = h->C.H0, L = h->C.lidar_n, PW = h->PW;
@@ -1180,10 +1244,11 @@ int64_t msv_kernel_bytes_per_env(msv_handle* h, int32_t which) {
   }
   if (which == 1) return 48 * A + 8 + om + 16 + 32 * B + 16 * B + 8 * H + 40 + h->obs_floats * 4;
   if (which == 2) return L > 0 ? 16 + 32 * B + 16 * B + 8 * H + 32 * A + 8 * A * L : 0;
+  if (which == 3) return h->gs_on ? 48 * A + 16 + 32 * B + 16 * B + 8 * H + 40 + 4 * (int64_t)h->gs.Ds : 0;
   return 0;
 }
 int64_t msv_bytes_per_env_step(msv_handle* h) {
-  return msv_kernel_bytes_per_env(h, 0) + msv_kernel_bytes_per_env(h, 1) + msv_kernel_bytes_per_env(h, 2);
+  return msv_kernel_bytes_per_env(h, 0) + msv_kernel_bytes_per_env(h, 1) + msv_kernel_bytes_per_env(h, 2) + msv_kernel_bytes_per_env(h, 3);
 }
 int64_t msv_obs_bytes_per_env(msv_handle* h) { return h ? h->obs_floats * 4 : 0; }
 int64_t msv_kernel_launches(msv_handle* h) { return h ? h->launches : 0; }

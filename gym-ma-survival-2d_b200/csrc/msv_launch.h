@@ -1,5 +1,5 @@
 // msv_launch.h -- host-side interface between the C ABI (msv_abi.cu) and the
-// kernel launchers (msv_kernels.cu, msv_render.cu).
+// kernel launchers (msv_kernels.cu, msv_render.cu, msv_state.cu).
 #pragma once
 #include "msv_types.cuh"
 #define MSV_TPB 512   // maximum threads per block of k_step / k_reset / k_observe (the actual size is a runtime choice, see plan_blocks)
@@ -39,3 +39,25 @@ struct RenderArgs {
 };
 cudaError_t msv_launch_render(const DevConst& C, const DevState& S, const DevOut& O, RenderArgs R, cudaStream_t st);
 int msv_palette(uint8_t* out_rgb, int capacity);   // copies min(capacity, n) colours, returns n
+
+// ---- global state (msv_state.cu) -------------------------------------------
+// The row of one environment, keys in this order (a key whose list the config lacks has width 0: no heal keys when
+// H = 0, no box keys when B = 0).  col[k] is key k's first column, Ds the row width.
+enum { GS_AGENTS, GS_AGENTS_MASK, GS_ZONE, GS_HEALS, GS_HEALS_MASK, GS_HEAL_SLOT, GS_HEAL_SLOT_MASK, GS_BOXES,
+       GS_BOXES_MASK, GS_BOX_ITEMS, GS_BOX_ITEMS_MASK, GS_BOX_SLOT, GS_BOX_SLOT_MASK, GS_STEPS, GS_KEYS };
+struct GsLayout { int col[GS_KEYS]; int Ds; };
+inline GsLayout gs_layout(int A, int B, int H, int S) {
+  const int hk = H > 0 ? 1 : 0, bk = B > 0 ? 1 : 0;
+  const int w[GS_KEYS] = {A * S, A, 6, hk * 2 * H, hk * H, hk * A, hk * A, bk * 11 * B, bk * B, bk * 10 * B, bk * B, bk * 8 * A, bk * A, 1};
+  GsLayout L;
+  int c = 0;
+  for (int k = 0; k < GS_KEYS; ++k) { L.col[k] = c; c += w[k]; }
+  L.Ds = c;
+  return L;
+}
+// one-time, on the current device: the dynamic shared memory k_global_state's stage needs (up to 52 KB)
+cudaError_t msv_global_state_attrs();
+// k_global_state into out ([C.N][Ds] floats): every row (only_if NULL), or the rows of the real envs whose
+// only_if byte is set
+cudaError_t msv_launch_global_state(const DevConst& C, const DevState& S, const GsLayout& Lg, float* out, const uint8_t* only_if,
+                                    cudaStream_t st);

@@ -22,7 +22,8 @@ EXPORTS = [
     'msv_step_host', 'msv_step_host_obs', 'msv_step_host_async', 'msv_step_host_wait', 'msv_obs_host_bytes',
     'msv_obs_host_offset', 'msv_device_bytes', 'msv_tensor', 'msv_tensor_info', 'msv_get_state', 'msv_set_state',
     'msv_observe', 'msv_flush_stats', 'msv_bytes_per_env_step', 'msv_kernel_bytes_per_env', 'msv_obs_bytes_per_env', 'msv_kernel_launches', 'msv_tile_plan', 'msv_plan_tile',
-    'msv_last_error', 'msv_philox4x32', 'msv_render', 'msv_render_palette',
+    'msv_last_error', 'msv_philox4x32', 'msv_render', 'msv_render_palette', 'msv_global_state_dim',
+    'msv_enable_global_state',
 ]
 
 MSV_RENDER_LIDAR = 1
@@ -43,6 +44,16 @@ def render_palette():
     if n < 0:
         check(n)
     return out[:n].copy()
+
+
+def global_state_dim(rec):
+    """Width Ds of the global-state row of config record `rec` (msv_global_state_dim; no device needed)."""
+    L = load()
+    buf = np.array(rec, dtype=CONFIG_DT).reshape(1)
+    n = L.msv_global_state_dim(buf.ctypes.data)
+    if n < 0:
+        check(n)
+    return int(n)
 
 
 _lib = None
@@ -102,6 +113,8 @@ def load():
     L.msv_philox4x32.argtypes = [vp, vp, vp]
     L.msv_render.argtypes = [vp, i32, i32, i32, i32, ctypes.c_uint32, vp, vp]
     L.msv_render_palette.argtypes = [vp, i32]
+    L.msv_global_state_dim.argtypes = [vp]
+    L.msv_enable_global_state.argtypes = [vp, vp]
     L.msv_debug_step_kernel.argtypes = [vp, vp, vp]
     L.msv_debug_obs_kernel.argtypes = [vp, vp]
     L.msv_debug_overflow.argtypes = [vp]
@@ -204,6 +217,10 @@ class Handle:
         check(load().msv_render(self.h, int(first), int(count), int(out.shape[1]), int(out.shape[2]), int(flags),
                                 out.data_ptr(), stream), self.h)
 
+    def enable_global_state(self, stream=0):
+        """msv_enable_global_state: from now on every call that writes observations also writes "global_state"."""
+        check(load().msv_enable_global_state(self.h, stream), self.h)
+
     def step_host(self, actions, rewards, dones, stream=0):
         check(load().msv_step_host(self.h, actions, rewards, dones, stream), self.h)
 
@@ -262,7 +279,7 @@ class Handle:
         return int(load().msv_bytes_per_env_step(self.h))
 
     def kernel_bytes_per_env(self, which):
-        """algorithmic HBM bytes per env-step of kernel `which` (0 k_step, 1 k_obs2, 2 k_lidar)"""
+        """algorithmic HBM bytes per env-step of kernel `which` (0 k_step, 1 k_obs2, 2 k_lidar, 3 k_global_state)"""
         return int(load().msv_kernel_bytes_per_env(self.h, which))
 
     def obs_bytes_per_env(self):

@@ -49,12 +49,20 @@ class MaSurvivalVec:
                             flat_obs_layout()), ready for a policy shared by
                             the agents; the observation dicts are the same,
                             as strided views into it
+    global_state : bool     True: the library also writes the global state of
+                            every environment, one float32 row of Ds floats
+                            (state(), state_layout(), state_space): what an
+                            omniscient observer sees, stored once, plus the
+                            alive mask and the step count -- the input of a
+                            centralised critic.  With auto_reset='terminal',
+                            step()'s info carries info['terminal_state'] (rows
+                            valid where the episode finished)
     """
 
     metadata = {'render_modes': ['rgb_array'], 'render_fps': 30}
 
     def __init__(self, config=None, num_envs=1, device=0, seed=0, env_offset=0, auto_reset=True, max_episode_steps=None,
-                 obs_layout='dict'):
+                 obs_layout='dict', global_state=False):
         self.config, self._continuous_melee = merge_config(config)
         self._rec = pack_config(self.config, self._continuous_melee, auto_reset=auto_reset,
                                 max_episode_steps=max_episode_steps or 0, obs_layout=obs_layout)
@@ -72,6 +80,9 @@ class MaSurvivalVec:
         self._trunc_bool = None
         self._host_obs = None
         self._mask_buf = None
+        self.global_state = bool(global_state)
+        if self.global_state:
+            self._h.enable_global_state(self._stream())
 
     # ---- reference properties (env:245-291) --------------------------------
     @property
@@ -157,6 +168,36 @@ class MaSurvivalVec:
         return {k: ((self._h.tensor_info(k)[0] - base) // 4, shp[1:])
                 for k, shp in self.obs_shapes().items() if k != 'lidar_hit'}
 
+    # ---- global state (PettingZoo's state() / state_space) ----------------------
+    # the row's keys, in column order; the heal keys exist only with heals, the box keys only with boxes
+    STATE_KEYS = ('agents', 'agents_mask', 'zone', 'heals', 'heals_mask', 'heal_slot', 'heal_slot_mask', 'boxes',
+                  'boxes_mask', 'box_items', 'box_items_mask', 'box_slot', 'box_slot_mask', 'steps')
+
+    @property
+    def state_space(self):
+        return spaces.Box(float('-inf'), float('inf'), shape=(_lib.global_state_dim(self._rec),))
+
+    def state(self):
+        """global_state=True: the float32 tensor [N, Ds] the library writes, row e = environment e's global
+        state (column ranges: state_layout()).  Zero-copy, the same storage on every call; like every output
+        it is valid until the next step / reset / observe."""
+        if not self.global_state:
+            raise RuntimeError('state() needs MaSurvivalVec(..., global_state=True)')
+        return self._h.tensor('global_state')
+
+    def state_layout(self):
+        """global_state=True: {key: (first column, shape)} in column order, read from the library's tensor
+        pointers (see STATE_KEYS and include/masurv.h)."""
+        if not self.global_state:
+            raise RuntimeError('state_layout() needs MaSurvivalVec(..., global_state=True)')
+        base = self._h.tensor_info('global_state')[0]
+        out = {}
+        for k in self.STATE_KEYS:
+            if self._h.has_tensor('global_state_' + k):
+                p, shape, _, _ = self._h.tensor_info('global_state_' + k)
+                out[k] = ((p - base) // 4, shape[1:])
+        return out
+
     def _stream(self):
         import torch
         return torch.cuda.current_stream(self.device).cuda_stream
@@ -234,6 +275,8 @@ class MaSurvivalVec:
         info = {'terminal_observation': self._obs('terminal_')} if self._terminal else {}
         if self._terminal and self.obs_layout == 'flat':
             info['terminal_observation_flat'] = self._h.tensor('terminal_obs_flat')
+        if self._terminal and self.global_state:
+            info['terminal_state'] = self._h.tensor('terminal_global_state')
         # per-env episode statistics (rows valid where done, or done | truncated under a step limit): what a
         # trainer logs at episode end
         info['episode_return'] = self._h.tensor('episode_return')
@@ -407,8 +450,12 @@ class MaSurvival(MaSurvivalVec):
     `reset()` -> dict of numpy float32 arrays, `step(actions)` ->
     `(obs, float32[A], bool, {})` with `actions` a tuple of A 6-tuples."""
 
-    def __init__(self, config=None, device=0, seed=0):
-        super().__init__(config, num_envs=1, device=device, seed=seed, auto_reset=False)
+    def __init__(self, config=None, device=0, seed=0, global_state=False):
+        super().__init__(config, num_envs=1, device=device, seed=seed, auto_reset=False, global_state=global_state)
+
+    def state(self):
+        """global_state=True: numpy float32[Ds], the environment's global state (see MaSurvivalVec.state)."""
+        return super().state()[0].cpu().numpy()
 
     def _np_obs(self, obs):
         return {k: v[0].cpu().numpy() for k, v in obs.items()}

@@ -358,13 +358,45 @@ int msv_render(msv_handle* h, int32_t first, int32_t count, int32_t height, int3
  * number of colours; out_rgb may be NULL when capacity is 0.  Needs no device. */
 int msv_render_palette(uint8_t* out_rgb, int32_t capacity);
 
+/* Global state for centralised critics: one float32 row of Ds floats per env,
+ * what an omniscient observer sees, stored once, plus an alive mask and the
+ * step count (no lidar).  Keys in this order; the heal keys exist only with
+ * n_heals > 0, the box keys only with n_boxes > 0; masks: 0 present, 1 absent.
+ *   agents [A][S]          obs['agent'][e] (id, (team), health, x, y, angle,
+ *                          vx, vy, omega; a dead agent keeps id and team)
+ *   agents_mask [A]        0 alive, 1 dead
+ *   zone [6]               obs['zone'][e]
+ *   heals [H][2], heals_mask [H]            0 where k < n_heals
+ *   heal_slot [A], heal_slot_mask [A]       obs['heal_slot'][e, i, 0, 0] and its mask
+ *   boxes [B][11], boxes_mask [B]           0 where k < n_boxes
+ *   box_items [B][10], box_items_mask [B]   0 where k < n_items
+ *   box_slot [A][8], box_slot_mask [A]      obs['box_slot'][e, i, 0] and its mask
+ *   steps [1]              the episode's step count (msv_env_state.steps)
+ * Ds = A*(S+1) + 6 + [H>0]*(3H + 2A) + [B>0]*(23B + 9A) + 1 (S = 8, 9 with teams).
+ * Width Ds of the row for cfg (host only, no device), or MSV_ERR_INVALID. */
+int msv_global_state_dim(const msv_config* cfg);
+/* Turn on the "global_state" output (float32 [num_envs][Ds]; with auto_reset 2
+ * also "terminal_global_state", rows valid where the episode finished on the
+ * last step, the other rows untouched).  Allocates the buffers, writes the row
+ * of every env for the current state on cuda_stream, and from then on every
+ * call that writes observations (step, reset, reset_envs, observe, the
+ * step_host forms) writes it too, after the observation kernels.  Each key is
+ * also exported as a strided view "global_state_<key>" (and
+ * "terminal_global_state_<key>"): shape [num_envs][key shape], stride Ds
+ * between envs; before the call these names are unknown (MSV_ERR_NAME).
+ * Idempotent (a second call rewrites the rows; pointers are unchanged).
+ * Refused (MSV_ERR_INVALID) for a NULL handle or while cuda_stream is being
+ * captured (it allocates).  The row is not part of the host read-back. */
+int msv_enable_global_state(msv_handle* h, void* cuda_stream);
+
 /* flush_stats (env:471-480) summed over all envs; zeroes the accumulators.
  * Synchronises the device first (work queued on any stream is complete). */
 int msv_flush_stats(msv_handle* h, msv_stats* out);
 
 /* Algorithmic HBM bytes one msv_step moves per env (state read+write,
  * actions, observations, rewards, dones) -- the roofline numerator -- and
- * its split by kernel (which: 0 step kernel, 1 observation gather, 2 lidar). */
+ * its split by kernel (which: 0 step kernel, 1 observation gather, 2 lidar,
+ * 3 global state: 0 until msv_enable_global_state). */
 int64_t msv_bytes_per_env_step(msv_handle* h);
 int64_t msv_kernel_bytes_per_env(msv_handle* h, int32_t which);
 /* The part of it written by the observation kernel (k_obs2). */
